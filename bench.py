@@ -10,6 +10,7 @@ guess 0.1.  One "step" = one batched solve of the whole batch (socp_solve_batch)
   python bench.py --impl reference ...                      (the reference's CPU solver, all cores)
   python bench.py --scaling strong --global-batch 1000000   (fixed total work split over the ranks)
   python bench.py --workload goddard_warm|interceptor|covid19|vtol_rk45   (the other BASELINE configs)
+  python bench.py --dump-outputs DIR ...                    (what the last timed step returned, as DIR/<name>.npy)
 
 Prints ONE JSON line (rank 0).  `value` = shooting solves per second with the inputs resident in HBM;
 `e2e` = the same through the public API with pinned HOST buffers (H2D + D2H inside the timed region);
@@ -59,6 +60,8 @@ def parse():
     ap.add_argument("--no-cpu-baseline", action="store_true", help="skip cpu_baseline, parity and stage2 parity")
     ap.add_argument("--no-stage2", action="store_true")
     ap.add_argument("--no-profile-pass", action="store_true")
+    ap.add_argument("--dump-outputs", metavar="DIR", default=None,
+                    help="write what the last timed step returned as DIR/<name>.npy (float64, at most 64 MB in all)")
     return ap.parse_args()
 
 
@@ -594,6 +597,43 @@ def timed_solves(eng, torch, dist, world, dev, w, d, steps, warmup, gather):
     return e0.elapsed_time(e1), step
 
 
+DUMP_BYTES = 64 * 10 ** 6          # --dump-outputs writes at most this much
+
+
+def step_outputs(w, d):
+    """The arrays a caller of the timed path receives after one unit of work (device tensors, one row per problem):
+    unknowns and status, |F| of a solve, the solver-call counts of a homotopy and the parameter block it rewrites."""
+    out = {"x": d["x"], "info": d["info"]}
+    if w.kind == "solve":
+        out.update(nfev=d["nfev"], fnorm=d["fnorm"])
+    else:
+        out["calls"] = d["calls"]
+    if w.kind == "cont_param":
+        out["mparams"] = d["mpw"]
+    return out
+
+
+def dump_outputs(torch, outputs, path):
+    """Write every output as <path>/<name>.npy in float64.  Where all of them together would exceed DUMP_BYTES, the
+    same fixed, seeded sample of problems is taken from each, and its row indices are written as sample_rows.npy."""
+    os.makedirs(path, exist_ok=True)
+    B = outputs["x"].shape[0]
+    if B == 0:                      # --scaling strong with fewer problems than ranks: this rank's block is empty
+        return 0
+    row_bytes = sum(8 * t.numel() // B for t in outputs.values())
+    n = min(B, (DUMP_BYTES - 4096) // (row_bytes + 8))         # 4 KB for the .npy headers
+    idx = None
+    if n < B:
+        rows = np.sort(np.random.default_rng(0).choice(B, n, replace=False))
+        np.save(os.path.join(path, "sample_rows.npy"), rows.astype(np.float64))
+        idx = torch.from_numpy(rows).to(outputs["x"].device)
+    for name, t in outputs.items():
+        if idx is not None:
+            t = t.index_select(0, idx)
+        np.save(os.path.join(path, name + ".npy"), t.to(torch.float64).cpu().numpy())
+    return n
+
+
 def e2e_solves(eng, torch, dist, world, dev, w, steps):
     """The same work through the C ABI with HOST buffers (mem = SOCP_HOST): pinned host memory, H2D and D2H inside the
     timed region (wall clock around the calls, max over ranks)."""
@@ -743,6 +783,11 @@ def main():
     st = eng.stats()
     sampler.stop_flag = True
     sampler.join(timeout=2)
+    if args.dump_outputs:
+        # the buffers still hold the last timed step: nothing has run since
+        path = args.dump_outputs if world == 1 else os.path.join(args.dump_outputs, "rank%d" % rank)
+        n = dump_outputs(torch, step_outputs(w, d), path)
+        print("outputs of the last timed step (%d of %d problems) written to %s" % (n, B, path), file=sys.stderr)
 
     if world > 1:
         print("rank %d: %.1f ms for %d step(s), %d solver rounds" % (rank, ms, args.steps, st["solver_rounds"]), file=sys.stderr)

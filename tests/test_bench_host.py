@@ -83,6 +83,43 @@ def test_strong_scaling_blocks_carry_every_per_problem_array():
                 assert s0["cont"]["step"] == w.cont["step"]
 
 
+def test_dump_outputs_writes_float64_within_budget(tmp_path):
+    """bench.py --dump-outputs: every output of the step as <name>.npy in float64; a batch too large for the budget
+    is sampled on the same fixed rows in every array, and the sample is the same from run to run."""
+    import torch
+    import bench
+    B, P = 200000, 85
+    w = bench.Workload("goddard", 0, None, None, None, None, np.zeros((B, P)), 1e-6, 10, "goddard", "", None, None, 6)
+    d = {"x": torch.arange(B * P, dtype=torch.float64).reshape(B, P), "info": torch.arange(B, dtype=torch.int32),
+         "nfev": torch.full((B,), 7, dtype=torch.int32), "fnorm": torch.zeros(B, dtype=torch.float64)}
+    outs = bench.step_outputs(w, d)
+    assert sorted(outs) == ["fnorm", "info", "nfev", "x"]
+    n = bench.dump_outputs(torch, outs, str(tmp_path / "a"))
+    assert 0 < n < B
+    files = sorted(os.listdir(tmp_path / "a"))
+    assert files == ["fnorm.npy", "info.npy", "nfev.npy", "sample_rows.npy", "x.npy"]
+    assert sum(os.path.getsize(tmp_path / "a" / f) for f in files) <= bench.DUMP_BYTES
+    rows = np.load(tmp_path / "a" / "sample_rows.npy").astype(np.int64)
+    x, info = np.load(tmp_path / "a" / "x.npy"), np.load(tmp_path / "a" / "info.npy")
+    assert x.dtype == np.float64 and info.dtype == np.float64 and x.shape == (n, P)
+    assert np.array_equal(info, rows) and np.array_equal(x[:, 0], rows * P)
+    bench.dump_outputs(torch, outs, str(tmp_path / "b"))
+    assert np.array_equal(np.load(tmp_path / "b" / "sample_rows.npy"), rows)
+    # a small batch is written whole; a homotopy returns its solver calls and the rewritten parameters
+    wc = bench.Workload("covid19", 2, None, None, None, None, np.zeros((8, 3)), 1e-6, 10, "covid19", "", None, None, 20,
+                        kind="cont_param")
+    dc = {"x": torch.ones(8, 3, dtype=torch.float64), "info": torch.ones(8, dtype=torch.int32),
+          "calls": torch.ones(8, 2, dtype=torch.int32), "mpw": torch.ones(8, 5, dtype=torch.float64)}
+    outs = bench.step_outputs(wc, dc)
+    assert sorted(outs) == ["calls", "info", "mparams", "x"]
+    assert bench.dump_outputs(torch, outs, str(tmp_path / "c")) == 8
+    assert "sample_rows.npy" not in os.listdir(tmp_path / "c")
+    assert np.load(tmp_path / "c" / "calls.npy").shape == (8, 2)
+    # an empty block (a rank of a strong-scaling run with fewer problems than ranks) writes nothing
+    outs = bench.step_outputs(wc, {k: v[:0] for k, v in dc.items()})
+    assert bench.dump_outputs(torch, outs, str(tmp_path / "e")) == 0 and os.listdir(tmp_path / "e") == []
+
+
 def test_ncu_traffic_record_belongs_to_these_sources():
     """roofline.traffic is taken from profiles/r2_traffic.json only when that record was captured from the CUDA sources
     being run (digest of socp_b200/csrc): the committed record must match the committed sources, and it must carry a
