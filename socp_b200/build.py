@@ -27,30 +27,14 @@ def stale(so=SO):
     return any(os.path.getmtime(s) > t for s in sources())
 
 
-def build_variant(name, extra):
-    """An A/B build with extra nvcc flags -> socp_b200/variants/<name>.so (select with SOCP_LIB)."""
-    d = os.path.join(HERE, "variants")
-    os.makedirs(d, exist_ok=True)
-    so = os.path.join(d, name + ".so")
-    cmd = [os.environ.get("NVCC", "nvcc")] + NVCC_FLAGS + list(extra) + ["-o", so, os.path.join(CSRC, "api.cu")]
-    r = subprocess.run(cmd, capture_output=True, text=True)
-    if r.returncode != 0:
-        sys.stderr.write(r.stdout + r.stderr)
-        raise RuntimeError("nvcc failed building " + so)
-    return so
-
-
-def build(force=False, verbose=False, extra=(), nofma=False):
+def build(force=False, verbose=False, nofma=False):
     """nvcc -gencode arch=compute_100a,code=sm_100a -lineinfo ... -> socp_b200/libsocp_b200.so
     (nofma=True: the -fmad=false parity build -> socp_b200/libsocp_b200_nofma.so)"""
     so = SO_NOFMA if nofma else SO
     if not force and not stale(so):
         return so
     nvcc = os.environ.get("NVCC", "nvcc")
-    extra = list(extra) + os.environ.get("SOCP_NVCC_EXTRA", "").split()      # experiments: -DSOCP_...=...
-    if nofma:
-        extra = extra + ["-fmad=false"]
-    cmd = [nvcc] + NVCC_FLAGS + list(extra) + (["-Xptxas", "-v"] if verbose else []) + \
+    cmd = [nvcc] + NVCC_FLAGS + (["-fmad=false"] if nofma else []) + (["-Xptxas", "-v"] if verbose else []) + \
           ["-o", so, os.path.join(CSRC, "api.cu")]
     r = subprocess.run(cmd, capture_output=True, text=True)
     if r.returncode != 0:

@@ -127,11 +127,9 @@ enum { SLOT_MPARAMS = 0, SLOT_SW, SLOT_T0, SLOT_TF, SLOT_X0, SLOT_XF, SLOT_AUX0,
        SLOT_CONT, SLOT_CONT_A, SLOT_CONT_B, SLOT_SOLVER_BASE };
 
 // cooperative groups (Coop<MODEL>::LANES lanes per trajectory) when one thread per trajectory cannot fill the GPU:
-// fewer threads than the device holds at the kernel's occupancy.  SOCP_COOP=0 / 1 forces never / always.
+// fewer threads than the device holds at the kernel's occupancy.
 static bool use_coop(socp_ctx *ctx, long items, int lanes) {
     if (lanes <= 1) return false;
-    static const char *env = getenv("SOCP_COOP");
-    if (env) return atoi(env) != 0;
     return items * lanes <= (long)ctx->sm_count * 128 * 4;
 }
 

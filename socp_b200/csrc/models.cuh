@@ -292,14 +292,9 @@ SOCP_DEV void obstacle_one(int i, double muObs, double imu, const double *pos, b
         // 1 - tanh(a) = 2 r and 1 - tanh(a)^2 = 4 r (1 - r) with r = 1 / (1 + exp(2a)): one exp and one
         // reciprocal per axis instead of a library tanh (exp + divide + range logic, ~2x the instructions)
         // and no cancellation in 1 - tanh far inside an obstacle's shadow; exp overflow gives r = 0, the limit
-#ifdef SOCP_OBS_TANH                       // A/B switch: the library tanh, as the reference writes it
-        double tx = tanh((fabs(dx) - radx) * imu), ty = tanh((fabs(dy) - rady) * imu), tz = tanh((fabs(dz) - radz) * imu);
-        double rx = (1 - tx) / 2, ry = (1 - ty) / 2, rz = (1 - tz) / 2;
-#else
         double rx = 1.0 / (1.0 + exp(2.0 * ((fabs(dx) - radx) * imu)));
         double ry = 1.0 / (1.0 + exp(2.0 * ((fabs(dy) - rady) * imu)));
         double rz = 1.0 / (1.0 + exp(2.0 * ((fabs(dz) - radz) * imu)));
-#endif
         double ax = 2.0 * rx, ay = 2.0 * ry, az = 2.0 * rz;
         a.f = a.f + ax * ay * az / 8;
         if (want_g) {
@@ -326,12 +321,6 @@ SOCP_DEV void obstacle_eval(double muObs, double phiObs, const double *pos, doub
         g0 = a.g0 + __shfl_xor_sync(cmask, a.g0, 2); g0 = g0 + __shfl_xor_sync(cmask, g0, 1);
         g1 = a.g1 + __shfl_xor_sync(cmask, a.g1, 2); g1 = g1 + __shfl_xor_sync(cmask, g1, 1);
         g2 = a.g2 + __shfl_xor_sync(cmask, a.g2, 2); g2 = g2 + __shfl_xor_sync(cmask, g2, 1);
-#ifdef SOCP_OBS_SEQ                        // A/B switch: one running sum over the obstacles (not the canonical order)
-    } else if (true) {
-        ObsAcc a = {0., 0., 0., 0.};
-        for (int i = 0; i < n; ++i) obstacle_one(i, muObs, imu, pos, func != nullptr, grad != nullptr, a);
-        f = a.f; g0 = a.g0; g1 = a.g1; g2 = a.g2;
-#endif
     } else {
         // the same four partial sums one after the other, in the order 0, 2, 1, 3 (one inlined copy of the
         // obstacle code, twelve live doubles): (s0 + s2) + (s1 + s3)
@@ -358,10 +347,7 @@ SOCP_DEV void obstacle_eval(double muObs, double phiObs, const double *pos, doub
 
 template <> struct Model<VTOL_UAV> {
     static constexpr int DIM = 6, N = 12, NP = 13, NCTRL = 3, DEFAULT_STEPS = 100;
-#ifndef SOCP_VTOL_MINB
-#define SOCP_VTOL_MINB 4
-#endif
-    static constexpr int MINB = SOCP_VTOL_MINB;      // 4: 128 registers, +45% throughput over 1 (occupancy hides the exp chains)
+    static constexpr int MINB = 4;      // 128 registers, +45% throughput over 1 (occupancy hides the exp chains)
     // coop_lanes / cq / cmask: the thread mapping of the obstacle sum (see obstacle_eval), set by the cooperative kernels
     struct Ctx { double umax, amax, alphaT, alphaV, invSigma, Vd, ca, phiObs, muObs; int coop_lanes, cq; unsigned cmask; };
     SOCP_DEV static void load(Ctx &c, const double *m, const double *) {
@@ -418,10 +404,7 @@ template <> struct Model<VTOL_UAV> {
 
 template <> struct Model<INTERCEPTOR> {
     static constexpr int DIM = 6, N = 12, NP = 17, NCTRL = 2, DEFAULT_STEPS = 50;
-#ifndef SOCP_ICPT_MINB
-#define SOCP_ICPT_MINB 4
-#endif
-    static constexpr int MINB = SOCP_ICPT_MINB;      // 4: 128 registers, +65% throughput over 1 (occupancy hides the sin/cos chains)
+    static constexpr int MINB = 4;      // 128 registers, +65% throughput over 1 (occupancy hides the sin/cos chains)
     struct Ctx {
         double c0, hr, d0, eta, mprop, mempty, q, ve, alphamax, umax, mugft, muT, muV, muC;
         int chart, stage;

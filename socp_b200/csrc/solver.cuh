@@ -66,8 +66,6 @@ struct SolverDev {
     const SolverDev *self;             // this struct in GLOBAL memory: what non-inlined device functions take by reference
                                        // (a reference to the kernel parameter would make every thread copy the 2.5 KB
                                        // struct to its local-memory frame)
-    int jac_fast;                      // Jacobian phase: 1 = qrfac_w / qform_w (four lanes per column; A/B only)
-    int jac_window;                    // Jacobian phase: 1 = register-window routines when the matrix has the block structure
     int sm_count;                      // multiprocessors of the device (seq_warp)
     int phase_clocks;                  // debugging aid (SOCP_PHASE_CLOCKS=1): accumulate clock64() per phase
 };
@@ -440,11 +438,9 @@ __global__ void __launch_bounds__(256) zero_fjac_kernel(SolverDev D, int cur) {
 // ---- kernel 2a: assemble residuals and forward-difference Jacobian columns ----------------------
 // One thread per residual request, one thread per (Jacobian request, column).  This is the only
 // solver kernel besides integrate_worklist that contains model code.
-#ifndef SOCP_ASM_MINB
-#define SOCP_ASM_MINB 3            // resident CTAs per SM asked of assemble_kernel (register cap 168; measured per 1e5-problem step: 191 ms uncapped at 230 registers, 174 ms at 168, 171 ms at 128 with more spills)
-#endif
+constexpr int ASM_MINB = 3;        // resident CTAs per SM asked of assemble_kernel (register cap 168; measured per 1e5-problem step: 191 ms uncapped at 230 registers, 174 ms at 168, 171 ms at 128 with more spills)
 template <int MODEL>
-__global__ void __launch_bounds__(128, SOCP_ASM_MINB)
+__global__ void __launch_bounds__(128, ASM_MINB)
 assemble_kernel(SolverDev D, int cur) {
     const int nres = D.counts[cur * 2 + 0], njac = D.analytic ? 0 : D.counts[cur * 2 + 1];
     const int *res_list = D.lists + (size_t)(cur * 2 + 0) * D.B;
@@ -840,142 +836,7 @@ __device__ void qrfac_g(int n, double *a, int lda, double *rdiag, double *acnorm
     }
 }
 
-// ---- the same two routines for a 128-thread CTA, built for latency: one CTA barrier per Householder step
-// (three / two above) and four lanes per column.
-// * Every warp forms the reflector of step j REDUNDANTLY from column j (norm, sign, scaling) into its own
-//   buffer -- same bits in every warp, no barrier between norm, scaling and application.  The scaled column is
-//   written back by one warp at the start of the next step, when nobody reads it any more.
-// * Application: a column is owned by FOUR lanes; lane q accumulates the elements e = q (mod 4) -- exactly the
-//   four running sums of dot4 -- and two shuffles form (s0 + s1) + (s2 + s3): the factors are bit for bit
-//   those of qrfac_g / qform_g (and so of the dense MINPACK loops, up to the sign of a zero).
-// vbuf: [2][G/32][n] doubles of shared memory (qform double-buffers the reflector).
-SOCP_DEV double quarter_partial(const double *v, const double *c, int len, int q) {
-    const int m4 = len & ~3;
-    double s = 0.;
-    for (int e = q; e < m4; e += 4) s = fma(v[e], c[e], s);
-    if (q == 0) for (int e = m4; e < len; ++e) s = fma(v[e], c[e], s);      // dot4 puts the tail on its first sum
-    return s;
-}
-// (s0 + s1) + (s2 + s3) over the four lanes of a column; executed by every lane of the warp at ONE site
-SOCP_DEV double quarter_reduce(double s) {
-    s += __shfl_xor_sync(0xffffffffu, s, 1);
-    s += __shfl_xor_sync(0xffffffffu, s, 2);
-    return s;
-}
-
-template <int G>
-__device__ void qrfac_w(int n, double *a, int lda, double *rdiag, double *acnorm, double *qtf, double *vbuf, int rot, int *hi) {
-    constexpr int NW = G / 32;
-    const int tid = (threadIdx.x + 32 * rot) % G;
-    const int warp = tid >> 5, lane = tid & 31, c = lane >> 2, q = lane & 3;
-    double *vb = vbuf + (size_t)warp * n;
-    gsync<G>();
-    for (int j = warp; j < n; j += NW) {               // column norms, one warp per column
-        const double v = enorm_warp(n, a + (size_t)j * lda);
-        if (lane == 0) acnorm[j] = v;
-    }
-    for (int k = tid; k <= n; k += G) {                // last non-zero row of every column (qtf: dense)
-        int last = (k < n) ? 0 : n - 1;
-        if (k < n) {
-            const double *ck = a + (size_t)k * lda;
-            for (int i = n - 1; i > 0; --i) if (ck[i] != 0.) { last = i; break; }
-        }
-        hi[k] = last;
-    }
-    gsync<G>();
-    int wb_j = -1, wb_len = 0;                         // reflector still to be written back into its column
-    for (int j = 0; j < n; ++j) {
-        if (wb_j >= 0 && warp == (wb_j % NW)) {        // nobody reads column wb_j below its diagonal any more
-            double *cw = a + (size_t)wb_j * lda + wb_j;
-            for (int e = lane; e < wb_len; e += 32) cw[e] = vb[e];
-        }
-        __syncwarp();
-        wb_j = -1;
-        double *cj = a + (size_t)j * lda;
-        const int hj = max(hi[j], j), len = hj - j + 1;
-        double ajnorm = enorm_warp(len, cj + j);
-        if (ajnorm != 0.) {
-            if (cj[j] < 0.) ajnorm = -ajnorm;
-            for (int e = lane; e < len; e += 32) {
-                double v = cj[j + e] / ajnorm;
-                if (e == 0) v += 1.;
-                vb[e] = v;
-            }
-            __syncwarp();
-            const double ajj = vb[0];
-            for (int k0 = j + 1 + warp * 8; k0 <= n; k0 += 8 * NW) {     // remaining columns, and qtf as column n
-                const int k = k0 + c;
-                const bool active = k <= n;
-                double *ck = (k < n) ? a + (size_t)k * lda + j : qtf + j;
-                const double sum = quarter_reduce(active ? quarter_partial(vb, ck, len, q) : 0.);
-                if (active && sum != 0.) {
-                    const double temp = sum / ajj;
-                    for (int e = q; e < len; e += 4) ck[e] = __fma_rn(-temp, vb[e], ck[e]);
-                    if (q == 0 && hi[k] < hj) hi[k] = hj;
-                }
-            }
-            wb_j = j; wb_len = len;
-        }
-        if (tid == 0) rdiag[j] = -ajnorm;
-        gsync<G>();
-    }
-    if (wb_j >= 0 && warp == (wb_j % NW)) {
-        double *cw = a + (size_t)wb_j * lda + wb_j;
-        for (int e = lane; e < wb_len; e += 32) cw[e] = vb[e];
-    }
-    gsync<G>();
-}
-
-template <int G>
-__device__ void qform_w(int n, double *qm, int lda, double *vbuf, int rot, const int *hi) {
-    constexpr int NW = G / 32;
-    const int tid = (threadIdx.x + 32 * rot) % G;
-    const int warp = tid >> 5, lane = tid & 31, c = lane >> 2, q = lane & 3;
-    for (int j = 1 + tid; j < n; j += G)
-        for (int i = 0; i < j; ++i) qm[i + (size_t)j * lda] = 0.;
-    // reflector k lives in column k, rows k..hk, and no step before its own touches it: every warp copies the
-    // NEXT reflector into its spare buffer before the barrier that ends a step, so the owner of column k may
-    // overwrite it (with H_k e_k) right after that barrier
-    {
-        const int k = n - 1, len = max(hi[k], k) - k + 1;
-        double *vb = vbuf + (size_t)warp * n;
-        for (int e = lane; e < len; e += 32) vb[e] = qm[(size_t)k * lda + k + e];
-    }
-    gsync<G>();
-    for (int l = 0; l < n; ++l) {
-        const int k = n - 1 - l;
-        const int hk = max(hi[k], k), len = hk - k + 1;
-        const double *vb = vbuf + ((size_t)(l & 1) * NW + warp) * n;
-        if (k > 0) {
-            const int k2 = k - 1, len2 = max(hi[k2], k2) - k2 + 1;
-            double *nb = vbuf + ((size_t)((l + 1) & 1) * NW + warp) * n;
-            for (int e = lane; e < len2; e += 32) nb[e] = qm[(size_t)k2 * lda + k2 + e];
-        }
-        const double wk = vb[0];
-        if (wk != 0.) {
-            for (int j0 = k + warp * 8; j0 < n; j0 += 8 * NW) {
-                const int j = j0 + c;
-                const bool active = j < n;
-                double *cj = qm + (size_t)j * lda + k;
-                // column k is e_k here (never stored): dot4's four sums are (w_k, 0, 0, 0), the update is e_k - (w_k / w_k) w
-                double part = 0.;
-                if (j == k) part = (q == 0) ? vb[0] : 0.;
-                else if (active) part = quarter_partial(cj, vb, len, q);
-                const double sum = quarter_reduce(part);
-                if (active && sum != 0.) {
-                    const double temp = sum / wk;
-                    if (j == k) for (int e = q; e < len; e += 4) cj[e] = __fma_rn(-temp, vb[e], (e == 0) ? 1. : 0.);
-                    else for (int e = q; e < len; e += 4) cj[e] = __fma_rn(-temp, vb[e], cj[e]);
-                }
-            }
-        } else if (warp == 0 && c == 0) {
-            for (int e = q; e < len; e += 4) qm[(size_t)k * lda + k + e] = (e == 0) ? 1. : 0.;
-        }
-        gsync<G>();
-    }
-}
-
-// ---- register-window Householder routines (block-bidiagonal + border Jacobians) ---------------------------------
+// ---- register-window accumulation of Q (block-bidiagonal + border Jacobians) ------------------------------------
 // The shooting Jacobian of a problem without free interior times is block bidiagonal (blocks of NB = 2 dim rows and
 // columns) plus a border, and Householder reflector k then spans at most the rows of TWO blocks: k .. c0(k) + W - 1,
 // c0(k) = NB (k / NB) the first column of its panel, W = 2 NB.  window_ok() checks exactly that on the matrix at hand
@@ -1071,123 +932,6 @@ __device__ void qform_p(int n, const double *a, int lda, const int *hi, double *
     }
 }
 
-//   qrfac_p : the factorisation itself, a panel of NB reflectors at a time.  Thread k holds the W window rows of
-//             column k (the columns c0 .. n-1 of the panel and to its right, and Q^T f as column n) in registers for the
-//             whole panel.  A step: the owner of column j publishes its raw sub-column; every warp forms its norm
-//             (enorm_warp on the published copy: the same bits in every warp, no barrier for it); len threads scale one
-//             element each; every column to the right applies the reflector to its window registers.  Two barriers per
-//             reflector, and the only shared-memory traffic is the published reflector (qrfac_g: three barriers, every
-//             operand of every column through shared memory).  Bit for bit the factors of qrfac_g.
-// pub: [2][2 W + 2] doubles of shared memory (raw sub-column, scaled reflector, the span of the sub-column).
-// dot4 of the published reflector with the window (compile-time window position: every index is a register)
-template <int W, int KK>
-SOCP_DEV double win_dot4(int len, const double *x, const double (&c)[W]) {
-    double s0 = 0., s1 = 0., s2 = 0., s3 = 0.;
-#pragma unroll
-    for (int g = 0; g < (W - KK + 3) / 4; ++g) {
-        constexpr int dummy = 0; (void)dummy;
-        const int t = KK + 4 * g;
-        if (4 * g + 3 < len) {
-            if (t + 3 < W) {
-                s0 = fma(x[t], c[t], s0); s1 = fma(x[t + 1], c[(t + 1 < W) ? t + 1 : 0], s1);
-                s2 = fma(x[t + 2], c[(t + 2 < W) ? t + 2 : 0], s2); s3 = fma(x[t + 3], c[(t + 3 < W) ? t + 3 : 0], s3);
-            }
-        } else {
-            if (4 * g < len && t < W) s0 = fma(x[t], c[t], s0);
-            if (4 * g + 1 < len && t + 1 < W) s0 = fma(x[t + 1], c[(t + 1 < W) ? t + 1 : 0], s0);
-            if (4 * g + 2 < len && t + 2 < W) s0 = fma(x[t + 2], c[(t + 2 < W) ? t + 2 : 0], s0);
-        }
-    }
-    return (s0 + s1) + (s2 + s3);
-}
-
-// one reflector of a panel (JJ: its position in the panel, a compile-time constant so that the window stays in registers)
-template <int G, int NB, int JJ>
-struct QrStep {
-    static constexpr int W = 2 * NB, PS = 2 * W + 2;
-    SOCP_DEV static void run(int n, int c0, int tid, int k, bool mine, double (&c)[2 * NB], double *pub, double *rdiag, int *hi) {
-        const int j = c0 + JJ;
-        if (j < n) {                                   // uniform
-            double *raw = pub + (size_t)(JJ & 1) * PS, *vs = raw + W;
-            if (tid == JJ) {                           // the owner of column j publishes its sub-column
-                // hi[j] is this thread's own entry (it alone updates it, when a reflector fills its column): nobody
-                // else may read it before the barrier, so the span travels with the published sub-column
-#pragma unroll
-                for (int t = JJ; t < W; ++t) raw[t] = c[t];
-                raw[2 * W] = (double)(max(hi[j], j) - j + 1);
-            }
-            gsync<G>();
-            const int len = (int)raw[2 * W], hj = j + len - 1;
-            double ajnorm = enorm_warp(len, raw + JJ);
-            if (ajnorm != 0.) {                        // uniform
-                if (raw[JJ] < 0.) ajnorm = -ajnorm;
-                // scaling: one element per thread (the same divide the thread-per-row loop of qrfac_g does)
-                if (tid < len) {
-                    double v = raw[JJ + tid] / ajnorm;
-                    if (tid == 0) v += 1.;
-                    vs[JJ + tid] = v;
-                }
-                gsync<G>();
-                if (tid == JJ) {
-#pragma unroll
-                    for (int t = JJ; t < W; ++t) if (t - JJ < len) c[t] = vs[t];
-                } else if (mine && tid > JJ) {
-                    const double ajj = vs[JJ];
-                    const double sum = win_dot4<W, JJ>(len, vs, c);
-                    if (sum != 0.) {
-                        const double temp = sum / ajj;
-#pragma unroll
-                        for (int t = JJ; t < W; ++t) if (t - JJ < len) c[t] = __fma_rn(-temp, vs[t], c[t]);
-                        if (hi[k] < hj) hi[k] = hj;
-                    }
-                }
-            }
-            if (tid == JJ) rdiag[j] = -ajnorm;
-        }
-        QrStep<G, NB, JJ + 1>::run(n, c0, tid, k, mine, c, pub, rdiag, hi);
-    }
-};
-template <int G, int NB>
-struct QrStep<G, NB, NB> {
-    SOCP_DEV static void run(int, int, int, int, bool, double (&)[2 * NB], double *, double *, int *) {}
-};
-
-template <int G, int NB>
-__device__ void qrfac_p(int n, double *a, int lda, double *rdiag, double *acnorm, double *qtf, double *pub, int *hi) {
-    constexpr int W = 2 * NB;
-    const int tid = threadIdx.x % G, lane = tid & 31;
-    gsync<G>();
-    for (int j = tid >> 5; j < n; j += G / 32) {       // column norms, one warp per column
-        const double v = enorm_warp(n, a + (size_t)j * lda);
-        if (lane == 0) acnorm[j] = v;
-    }
-    for (int k = tid; k <= n; k += G) {                // last non-zero row of every column (qtf: dense)
-        int last = (k < n) ? 0 : n - 1;
-        if (k < n) {
-            const double *ck = a + (size_t)k * lda;
-            for (int i = n - 1; i > 0; --i) if (ck[i] != 0.) { last = i; break; }
-        }
-        hi[k] = last;
-    }
-    gsync<G>();
-    const int npan = (n + NB - 1) / NB;
-#pragma unroll 1
-    for (int p = 0; p < npan; ++p) {
-        const int c0 = p * NB;
-        const int k = c0 + tid;                        // this thread's column (k == n: Q^T f); idle beyond
-        const bool mine = k <= n;
-        double *col = (k < n) ? a + (size_t)k * lda : qtf;
-        double c[W];
-#pragma unroll
-        for (int t = 0; t < W; ++t) c[t] = (mine && c0 + t < n) ? col[c0 + t] : 0.;
-        QrStep<G, NB, 0>::run(n, c0, tid, k, mine, c, pub, rdiag, hi);
-        // windows back to shared memory; the next panel's columns read rows c0 + NB .. from there
-#pragma unroll
-        for (int t = 0; t < W; ++t) if (mine && c0 + t < n) col[c0 + t] = c[t];
-        gsync<G>();
-    }
-}
-
 // copy R into packed storage (upper triangle by rows), diagonal from rdiag
 template <int G>
 __device__ void pack_r_g(int n, const double *a, int lda, const double *rdiag, double *r) {
@@ -1240,38 +984,6 @@ __device__ void rmulv_g(int n, const double *r, const double *v, const double *a
     gsync<G>();
 }
 
-// The same product for a packed factor that lives in GLOBAL memory (one warp per problem, 16 problems per SM):
-// a row per step with the lanes along it -- consecutive lanes, consecutive addresses -- and a butterfly per row;
-// four rows are in flight so that the shuffle latencies overlap.  (The thread-per-row form above touches 32
-// different lines per load when R is not in shared memory.)
-SOCP_DEV void rmulv_rows(int n, const double *r, const double *v, const double *add, double *y) {
-    const int lane = threadIdx.x & 31;
-    __syncwarp();
-    for (int i0 = 0; i0 < n; i0 += 4) {
-        double p[4];
-#pragma unroll
-        for (int u = 0; u < 4; ++u) {
-            const int i = i0 + u;
-            p[u] = 0.;
-            if (i < n) {
-                const double *row = r + rowstart(n, i);
-                const int len = n - i;
-                for (int t = lane; t < len; t += 32) p[u] = fma(row[t], v[i + t], p[u]);
-            }
-        }
-#pragma unroll
-        for (int off = 16; off > 0; off >>= 1) {
-#pragma unroll
-            for (int u = 0; u < 4; ++u) p[u] += __shfl_xor_sync(0xffffffffu, p[u], off);
-        }
-        if (lane < 4 && i0 + lane < n) {
-            const double s = (lane == 0) ? p[0] : (lane == 1) ? p[1] : (lane == 2) ? p[2] : p[3];
-            y[i0 + lane] = (add ? add[i0 + lane] : 0.) + s;
-        }
-    }
-    __syncwarp();
-}
-
 // steps j = min(32 PH + 31, n - 1) .. 32 PH of dogleg's back substitution for n <= 96 (see dogleg_g)
 template <int PH>
 SOCP_DEV void backsub_phase(int n, const double *r, const double *dinvs, const double *ds, int lane,
@@ -1292,7 +1004,7 @@ SOCP_DEV void backsub_phase(int n, const double *r, const double *dinvs, const d
 }
 
 // dogleg: x <- step; wa1, wa2 scratch
-template <int G, bool RROWS = false>
+template <int G>
 __device__ void dogleg_g(int n, const double *r, const double *diag, const double *qtb, double delta,
                          double *x, double *wa1, double *wa2, double *red, int seqw, bool clk_on = false,
                          unsigned long long *clk_counters = nullptr) {
@@ -1369,8 +1081,7 @@ __device__ void dogleg_g(int n, const double *r, const double *diag, const doubl
     if (gnorm != 0.) {
         gsync<G>();
         for (int j = tid; j < n; j += G) wa1[j] = (wa1[j] / gnorm) / diag[j];
-        if (RROWS) rmulv_rows(n, r, wa1, nullptr, wa2);
-        else rmulv_g<G>(n, r, wa1, nullptr, wa2);
+        rmulv_g<G>(n, r, wa1, nullptr, wa2);
         double temp = enorm_g<G>(n, wa2, red);
         sgnorm = (gnorm / temp) / temp;
         alpha = 0.;
@@ -1851,12 +1562,12 @@ struct Work {
 };
 
 // dogleg step from the current factors, trial point xe = x + p, and the request for F(xe)
-template <int G, bool RROWS = false>
+template <int G>
 __device__ void dogleg_and_request(const SolverDev &D, long b, const Work &W, int *is, double *ds, double *red,
                                    int *next_res, int *next_cnt) {
     const int n = D.P, tid = threadIdx.x % G;
     const double delta = ds[D_DELTA];
-    dogleg_g<G, RROWS>(n, W.r, W.diag, W.qtf, delta, W.wa1, W.wa2, W.wa3, red, seq_warp<G>(D.sm_count), D.phase_clocks, D.counters);
+    dogleg_g<G>(n, W.r, W.diag, W.qtf, delta, W.wa1, W.wa2, W.wa3, red, seq_warp<G>(D.sm_count), D.phase_clocks, D.counters);
     for (int j = tid; j < n; j += G) {
         const double pj = -W.wa1[j];
         W.wa1[j] = pj;
@@ -1889,6 +1600,7 @@ SOCP_DEV double *group_smem(const SolverDev &D, int per_group_doubles) {
 // (I_PEND) and only qtf is rotated on the spot.
 template <int G, bool STAGE_R, bool SPLIT>
 SOCP_DEV void res_loop(const SolverDev &D, int cur, int per_group_doubles) {
+    static_assert(!SPLIT || (G == 32 && STAGE_R), "the chain kernel runs one warp per problem with R staged");
     const int GROUPS = (G == 32) ? (int)(blockDim.x >> 5) : 1;
     const int grp = (G == 32) ? (threadIdx.x >> 5) : 0;
     const int tid = threadIdx.x % G;
@@ -1931,10 +1643,10 @@ SOCP_DEV void res_loop(const SolverDev &D, int cur, int per_group_doubles) {
         // ---- trial point evaluated: wa4 = F(x + p) ----
         long long phase_t0 = clock64();
         Work W;
-        // LEAN (the chain kernel with R staged): only what the dependent chains touch lives in shared memory --
+        // LEAN (the chain kernel): only what the dependent chains touch lives in shared memory --
         // R and nine vectors; x, xe, fvec and F(x + p) are read and written element-wise and stay in global
         // memory.  35 KB per problem instead of 38: six problems per SM instead of five.  R travels by bulk copy.
-        constexpr bool LEAN = SPLIT && STAGE_R && G == 32;
+        constexpr bool LEAN = SPLIT;
         if (LEAN) {
             W.x = D.x + b * n; W.xe = D.xe + b * n; W.fvec = D.fvec + b * n; W.wa4 = D.wa4 + b * n;
             W.diag = vec; W.qtf = vec + n; W.wa1 = vec + 2 * n; W.wa2 = vec + 3 * n; W.wa3 = vec + 4 * n; W.scr = vec + 5 * n;
@@ -1981,9 +1693,7 @@ SOCP_DEV void res_loop(const SolverDev &D, int cur, int per_group_doubles) {
         double actred = -1.;
         if (fnorm1 < fnorm) { const double q = fnorm1 / fnorm; actred = 1. - q * q; }
         // predicted reduction: wa3 = qtf + R * wa1
-        constexpr bool RROWS = SPLIT && !STAGE_R && G == 32;
-        if (RROWS) rmulv_rows(n, W.r, W.wa1, W.qtf, W.wa3);
-        else rmulv_g<G>(n, W.r, W.wa1, W.qtf, W.wa3);
+        rmulv_g<G>(n, W.r, W.wa1, W.qtf, W.wa3);
         const double temp = enorm_g<G>(n, W.wa3, red);
         double prered = 0.;
         if (temp < fnorm) { const double q = temp / fnorm; prered = 1. - q * q; }
@@ -2132,7 +1842,7 @@ SOCP_DEV void res_loop(const SolverDev &D, int cur, int per_group_doubles) {
             } else r1mpyq_g<G>(n, n, W.q, W.ldq, W.scr, W.qtf);
             SOCP_PHASE(16, 5);
             if (tid == 0) is[I_JEVAL] = 0;
-            dogleg_and_request<G, RROWS>(D, b, W, is, ds, red, next_res, next_cnt);
+            dogleg_and_request<G>(D, b, W, is, ds, red, next_res, next_cnt);
             store_r = true;
             SOCP_PHASE(16, 6);
         }
@@ -2152,7 +1862,7 @@ SOCP_DEV void res_loop(const SolverDev &D, int cur, int per_group_doubles) {
         gsync<G>();
         SOCP_PHASE(16, 7);
     }
-    if (SPLIT && STAGE_R && G == 32 && tid == 0) bulk_wait_all();
+    if (SPLIT && tid == 0) bulk_wait_all();
 }
 
 // 4 CTAs/SM: after the instruction-level pass the kernel fits 128 registers without spills and the fourth
@@ -2168,10 +1878,9 @@ hybrd_res_kernel(SolverDev D, int cur, int per_group_doubles) {
 // __syncwarp), as many problems per SM as shared memory holds (R + 13 work vectors per problem).  What is left
 // of a Broyden iteration once Q is gone are the dependent chains (Givens sweeps, back substitution, norms);
 // their latency is hidden by the other warps of the SM instead of by idle threads of the same CTA.
-template <bool STAGE_R>
-__global__ void __launch_bounds__(32, STAGE_R ? 5 : 16)
+__global__ void __launch_bounds__(32, 5)
 hybrd_chain_kernel(SolverDev D, int cur, int per_group_doubles) {
-    res_loop<32, STAGE_R, true>(D, cur, per_group_doubles);
+    res_loop<32, true, true>(D, cur, per_group_doubles);
 }
 
 // ---- kernel 2c: problems whose forward-difference Jacobian arrived ------------------------------
@@ -2190,13 +1899,7 @@ hybrd_jac_kernel(SolverDev D, int cur, int per_group_doubles) {
     int *next_res = D.lists + (size_t)((1 - cur) * 2 + 0) * D.B;
     int *next_cnt = D.counts + (1 - cur) * 2;
     const int ldq_s = n | 1;                               // odd leading dimension in shared memory
-    // fast form (128-thread CTA, Q staged): Q travels by bulk copy when its shared layout equals the global
-    // one (odd P), the reflector buffers of qrfac_w / qform_w follow Q in shared memory
-#ifdef SOCP_JAC_LANES4
-    const bool fast = (G == 128) && STAGE_Q && D.jac_fast;      // A/B build only: four lanes per column (measured slower)
-#else
-    constexpr bool fast = false;
-#endif
+    // 128-thread CTA, Q staged: Q travels by bulk copy when its shared layout equals the global one (odd P)
     const bool bulk = (G == 128) && STAGE_Q && ldq_s == n;
     __shared__ unsigned long long jac_bar;
     unsigned jac_parity = 0;
@@ -2226,8 +1929,6 @@ hybrd_jac_kernel(SolverDev D, int cur, int per_group_doubles) {
         W.ldq = STAGE_Q ? ldq_s : n;
         long long phase_t0 = clock64();
         gcopy_async<G>(W.x, D.x + b * n, n); gcopy_async<G>(W.fvec, D.fvec + b * n, n); gcopy_async<G>(W.diag, D.diag + b * n, n);
-        double *vbuf = nullptr;
-        if (STAGE_Q) vbuf = W.q + (((size_t)ldq_s * n + 1) & ~(size_t)1);      // [2][G/32][n] reflector buffers (fast form)
         if (bulk) {
             if (tid == 0) {
                 bulk_wait_read();                          // the previous problem's copy out has read the buffer
@@ -2254,12 +1955,12 @@ hybrd_jac_kernel(SolverDev D, int cur, int per_group_doubles) {
         for (int i = tid; i < n; i += G) W.qtf[i] = W.fvec[i];
         // wa1 = rdiag, wa2 = acnorm
         int *hi = (int *)W.scr;                            // [n + 1] last non-zero row per column (scr is free here)
-        // Register-window routines when the Jacobian at hand has the block-bidiagonal + border structure (every
-        // sub-column fits the two-block window; fill-in stays inside it): decided per matrix, from its own zeros.
+        // Register-window accumulation of Q when the Jacobian at hand has the block-bidiagonal + border structure
+        // (every sub-column fits the two-block window; fill-in stays inside it): decided per matrix, from its own zeros.
         bool win = false;
         // (instantiated for the layout the 32 < P <= ~150 problems run with -- Q staged, R in global memory -- and the
-        // block size of the benchmark model, 14; every other shape takes the barrier-per-reflector routines)
-        if ((G == 128) && STAGE_Q && !STAGE_R && D.jac_window && D.N == 14 && n < G) {
+        // block size of the benchmark model, 14; every other shape takes the barrier-per-reflector qform_g)
+        if ((G == 128) && STAGE_Q && !STAGE_R && D.N == 14 && n < G) {
             for (int k = tid; k < n; k += G) {
                 const double *ck = W.q + (size_t)k * W.ldq;
                 int last = 0;
@@ -2268,17 +1969,6 @@ hybrd_jac_kernel(SolverDev D, int cur, int per_group_doubles) {
             }
             win = window_ok<G>(n, D.N, hi, (int *)red);
         }
-#ifdef SOCP_QRFAC_WINDOW
-        // the register-window factorisation: bit-identical, measured SLOWER than qrfac_g (351 k vs ~280 k cycles per
-        // Jacobian at P = 85, profiles/r2i_*): compiled only on request, for A/B runs
-        if ((G == 128) && STAGE_Q && !STAGE_R && win) {
-            qrfac_p<G, 14>(n, W.q, W.ldq, W.wa1, W.wa2, W.qtf, vbuf, hi);
-        } else
-#endif
-#ifdef SOCP_JAC_LANES4
-        if (fast) qrfac_w<G>(n, W.q, W.ldq, W.wa1, W.wa2, W.qtf, vbuf, seq_warp<G>(D.sm_count), hi);
-        else
-#endif
         qrfac_g<G>(n, W.q, W.ldq, W.wa1, W.wa2, W.qtf, red, seq_warp<G>(D.sm_count), hi);
         SOCP_PHASE(32, 1);
         if (is[I_ITER] == 1) {
@@ -2304,11 +1994,7 @@ hybrd_jac_kernel(SolverDev D, int cur, int per_group_doubles) {
             qform_p<G, 14>(n, W.q, W.ldq, hi, gq);
             gsync<G>();
             q_in_global = true;
-        }
-#ifdef SOCP_JAC_LANES4
-        else if (fast) qform_w<G>(n, W.q, W.ldq, vbuf, seq_warp<G>(D.sm_count), hi);
-#endif
-        else qform_g<G>(n, W.q, W.ldq, W.wa1, seq_warp<G>(D.sm_count), hi);
+        } else qform_g<G>(n, W.q, W.ldq, W.wa1, seq_warp<G>(D.sm_count), hi);
         SOCP_PHASE(32, 3);
         for (int j = tid; j < n; j += G) W.diag[j] = fmax(W.diag[j], W.wa2[j]);
         gsync<G>();

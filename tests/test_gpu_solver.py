@@ -239,6 +239,32 @@ def test_warm_started_batch_matches_reference_problem_for_problem(oracle_lib):
     assert np.all(r["fnorm"] < 1e-5)
 
 
+def test_solves_past_the_q_pass_limit_match_reference(oracle_lib):
+    """Goddard with free final time at M = 12 (P = 169): Q no longer fits one CTA's shared memory for the Q pass, so
+    the Broyden phase runs as one kernel per iteration (hybrd_res_kernel<128> with R staged) and the Jacobian phase
+    keeps Q in global memory.  Perturbed problems, each started from the converged M = 6 trajectory sampled at
+    twelve nodes, against the oracle ensemble."""
+    from backends import OracleBackend
+    from golden_util import by_name
+    ora = OracleBackend()
+    traj = lambda mp, t0, X0, tf: ora.traj(S.GODDARD, mp, t0, X0, tf, 10)
+    xs = np.asarray(unhex(by_name("solve", "goddard_stage1")["x"]))      # node 0 state + costates, ..., tf
+    Xi, xf0 = S.goddard_batch_inputs(4)
+    specs = []
+    for k in range(4):
+        spec = S.goddard_problem(traj, M=12, Xi=Xi[k], xf0=xf0[k])
+        time, x0 = S.init_guess(lambda t0, X0, tf: traj(spec["mparams"], t0, X0, tf), S.GODDARD, 12, 0.0, xs[:14], xs[-1],
+                                spec["mode_t"])
+        spec["time"], spec["x0"] = [float(v) for v in time], [float(v) for v in x0]
+        specs.append(spec)
+    assert S.num_param(specs[0]) == 169
+    r = gpu_solve(specs)
+    for k, spec in enumerate(specs):
+        runs = oracle_ensemble(ora.solve, spec)
+        check_against_ensemble("goddard_M12_%d" % k, spec, int(r["info"][k]), int(r["nfev"][k]), r["x"][k], runs)
+        assert r["info"][k] == 1 and r["fnorm"][k] <= 1e-4
+
+
 def test_kd_continuation_batch_matches_reference_outcome(oracle_lib):
     """SURVEY C2 stage 2, second half: continuation KD 0 -> 310 in one step (tests/testGoddard.cpp:105) from the
     warm-started solutions.  At KD = 310 the costates grow to 1e5..1e8 and the reference's own nfev moves with

@@ -18,7 +18,7 @@ base = {0: S.GODDARD_XI, 1: np.r_[np.zeros(6), 0.01*np.ones(6)], 2: S.COVID_XI,
 tfs = {0: 0.1, 1: 8.0, 2: 1.5, 3: 5.0, 4: 10.0}
 rng = np.random.default_rng(0)
 only = [int(v) for v in sys.argv[2].split(",")] if len(sys.argv) > 2 else list(range(5))     # model ids, e.g. "3" = vtolUAV
-print(json.dumps(dict(lib=os.environ.get("SOCP_LIB", "default"), coop=os.environ.get("SOCP_COOP", "auto"))))
+print(json.dumps(dict(lib=os.environ.get("SOCP_LIB", "default"))))
 for model in only:
     Bm = B if model != 2 else B // 16
     mp = np.array(S.DEFAULTS[model]);
