@@ -22,9 +22,33 @@ using namespace socp;
 namespace {
 std::string g_create_error;
 
-const int kDim[SOCP_NUM_MODELS] = {7, 6, 4, 6, 6};
-const int kNP[SOCP_NUM_MODELS] = {8, 3, 8, 13, 17};
-const int kSteps[SOCP_NUM_MODELS] = {10, 30, 1000, 100, 50};
+// Calls f(std::integral_constant<int, MODEL>) with the compile-time model of a valid SOCP_* model id.
+template <typename F>
+void with_model(int id, F &&f) {
+    switch (id) {
+    case SOCP_GODDARD: f(std::integral_constant<int, GODDARD>()); break;
+    case SOCP_DOUBLE_INTEGRATOR: f(std::integral_constant<int, DOUBLE_INTEGRATOR>()); break;
+    case SOCP_COVID19: f(std::integral_constant<int, COVID19>()); break;
+    case SOCP_VTOL_UAV: f(std::integral_constant<int, VTOL_UAV>()); break;
+    case SOCP_INTERCEPTOR: f(std::integral_constant<int, INTERCEPTOR>()); break;
+    }
+}
+
+bool valid_model(int id) { return id >= 0 && id < SOCP_NUM_MODELS; }
+
+struct ModelFacts {
+    int dim, np, steps;
+    int trace_width;                     // a trace row as trace_kernel writes it: t, X[N], control[NCTRL], H, extra
+};
+ModelFacts model_facts(int id) {
+    ModelFacts f{};
+    with_model(id, [&](auto m) {
+        using Mo = Model<decltype(m)::value>;
+        f = {Mo::DIM, Mo::NP, Mo::DEFAULT_STEPS, Mo::N + Mo::NCTRL + 3};
+    });
+    return f;
+}
+
 const double kPi = 3.14159265358979323846;
 const double kDefaults[SOCP_NUM_MODELS][17] = {
     {3.5, 7.0, 310.0, 500.0, 1.0, 1.0, 0.0, -1.0},                       // goddard.hpp:29-36
@@ -77,6 +101,25 @@ static int fail(socp_ctx *ctx, int code, const std::string &msg) {
     return code;
 }
 
+// error return after host buffers may have been staged: no asynchronous copy from (or to) a caller buffer
+// is left in flight when the call returns an error
+static int bail(socp_ctx *ctx, int rc) {
+    if (ctx) cudaStreamSynchronize(ctx->stream);
+    return rc;
+}
+
+// SOCP_ERR_CUDA, with the error text in ctx->err, when a launch (or an earlier runtime call) of this thread failed
+static int last_launch(socp_ctx *ctx) {
+    CUDA_TRY(ctx, cudaGetLastError());
+    return SOCP_OK;
+}
+
+// the last step of a batch call: with host buffers, the outputs have arrived when it returns
+static int finish(socp_ctx *ctx, int mem) {
+    if (mem == SOCP_HOST) CUDA_TRY(ctx, cudaStreamSynchronize(ctx->stream));
+    return SOCP_OK;
+}
+
 // workspace slot `slot` with at least `bytes` bytes
 static void *ws(socp_ctx *ctx, size_t slot, size_t bytes) {
     if (ctx->pool.size() <= slot) ctx->pool.resize(slot + 1);
@@ -126,6 +169,18 @@ enum { SLOT_MPARAMS = 0, SLOT_SW, SLOT_T0, SLOT_TF, SLOT_X0, SLOT_XF, SLOT_AUX0,
        SLOT_TIME, SLOT_XB, SLOT_X, SLOT_FVEC, SLOT_FJAC, SLOT_INFO, SLOT_NFEV, SLOT_FNORM, SLOT_PEAK,
        SLOT_CONT, SLOT_CONT_A, SLOT_CONT_B, SLOT_SOLVER_BASE };
 
+// The inputs of the trajectory-family calls on the device: mparams [B][np], sw [B][2], t0 [B], tf [B] and
+// X0 [B][nx] (null where the call has no such input).
+struct TrajIn {
+    const double *mp, *sw, *t0, *tf, *X0;
+};
+static TrajIn stage_traj(socp_ctx *ctx, long B, int np, int nx, const double *mparams, const double *sw,
+                         const double *t0, const double *tf, const double *X0, int mem, int *rc) {
+    return {stage_in(ctx, SLOT_MPARAMS, mparams, (size_t)B * np, mem, rc), stage_in(ctx, SLOT_SW, sw, (size_t)B * 2, mem, rc),
+            stage_in(ctx, SLOT_T0, t0, (size_t)B, mem, rc), stage_in(ctx, SLOT_TF, tf, (size_t)B, mem, rc),
+            stage_in(ctx, SLOT_X0, X0, (size_t)B * nx, mem, rc)};
+}
+
 // cooperative groups (Coop<MODEL>::LANES lanes per trajectory) when one thread per trajectory cannot fill the GPU:
 // fewer threads than the device holds at the kernel's occupancy.
 static bool use_coop(socp_ctx *ctx, long items, int lanes) {
@@ -134,61 +189,67 @@ static bool use_coop(socp_ctx *ctx, long items, int lanes) {
 }
 
 template <int MODEL>
-static void launch_traj(socp_ctx *ctx, long B, int S, const double *mp, const double *sw, const double *t0,
-                        const double *tf, const double *X0, double *Xf, double tol = 0., int *nsteps = nullptr) {
+static void launch_traj(socp_ctx *ctx, long B, int S, const TrajIn &in, double *Xf, double tol, int *nsteps) {
     const int threads = SOCP_TRAJ_THREADS;
     constexpr int L = Coop<MODEL>::LANES;
     if (use_coop(ctx, B, L)) {
         const long blocks = (B * L + threads - 1) / threads;
         if (tol > 0.)
-            traj_kernel<MODEL, true, L><<<(unsigned)blocks, threads, 0, ctx->stream>>>(B, S, mp, sw, t0, tf, X0, Xf, ctx->d_counters, tol, nsteps);
+            traj_kernel<MODEL, true, L><<<(unsigned)blocks, threads, 0, ctx->stream>>>(B, S, in.mp, in.sw, in.t0, in.tf, in.X0, Xf, ctx->d_counters, tol, nsteps);
         else
-            traj_kernel<MODEL, false, L><<<(unsigned)blocks, threads, 0, ctx->stream>>>(B, S, mp, sw, t0, tf, X0, Xf, ctx->d_counters, 0., nullptr);
+            traj_kernel<MODEL, false, L><<<(unsigned)blocks, threads, 0, ctx->stream>>>(B, S, in.mp, in.sw, in.t0, in.tf, in.X0, Xf, ctx->d_counters, 0., nullptr);
         ctx->launches += 1;
         return;
     }
     long blocks = (B + threads - 1) / threads;
     if (tol > 0.)
-        traj_kernel<MODEL, true><<<(unsigned)blocks, threads, 0, ctx->stream>>>(B, S, mp, sw, t0, tf, X0, Xf, ctx->d_counters, tol, nsteps);
+        traj_kernel<MODEL, true><<<(unsigned)blocks, threads, 0, ctx->stream>>>(B, S, in.mp, in.sw, in.t0, in.tf, in.X0, Xf, ctx->d_counters, tol, nsteps);
     else
-        traj_kernel<MODEL, false><<<(unsigned)blocks, threads, 0, ctx->stream>>>(B, S, mp, sw, t0, tf, X0, Xf, ctx->d_counters, 0., nullptr);
+        traj_kernel<MODEL, false><<<(unsigned)blocks, threads, 0, ctx->stream>>>(B, S, in.mp, in.sw, in.t0, in.tf, in.X0, Xf, ctx->d_counters, 0., nullptr);
     ctx->launches += 1;
 }
 
-template <int MODEL>
-static void launch_trace(socp_ctx *ctx, long B, int S, int max_rows, const double *mp, const double *sw, const double *t0,
-                         const double *tf, const double *X0, double *rows, int *nrows, double *Xf) {
-    trace_kernel<MODEL><<<(unsigned)((B + 63) / 64), 64, 0, ctx->stream>>>(B, S, max_rows, mp, sw, t0, tf, X0, rows, nrows, Xf);
-    ctx->launches += 1;
-}
-
-template <int MODEL>
-static void launch_point(socp_ctx *ctx, long B, const double *mp, const double *sw, const int *cs, const double *t,
-                         const double *X, double *rhs, double *control, double *H) {
-    const int threads = 128;
-    point_kernel<MODEL><<<(unsigned)((B + threads - 1) / threads), threads, 0, ctx->stream>>>(B, mp, sw, cs, t, X, rhs, control, H);
-    ctx->launches += 1;
+// fixed-step (tol = 0) or adaptive (tol > 0) trajectories; `what` names the entry point in the error text
+static int traj_batch(socp_ctx *ctx, const char *what, int model_id, int step_nbr, long B, const double *mparams,
+                      const double *sw, const double *t0, const double *tf, const double *X0, double tol, double *Xf,
+                      int *nsteps, int mem) {
+    if (!ctx) return SOCP_ERR_ARG;
+    if (!valid_model(model_id) || B < 0 || !mparams || !t0 || !tf || !X0 || !Xf)
+        return fail(ctx, SOCP_ERR_ARG, std::string(what) + ": bad arguments");
+    if (B == 0) return SOCP_OK;
+    CUDA_TRY(ctx, cudaSetDevice(ctx->device));
+    const ModelFacts m = model_facts(model_id);
+    const int N = 2 * m.dim, S = step_nbr > 0 ? step_nbr : m.steps;
+    int rc = SOCP_OK;
+    const TrajIn in = stage_traj(ctx, B, m.np, N, mparams, sw, t0, tf, X0, mem, &rc);
+    double *d_Xf = stage_out(ctx, SLOT_XF, Xf, (size_t)B * N, mem, &rc);
+    int *d_ns = stage_out(ctx, SLOT_INFO, nsteps, (size_t)B * 2, mem, &rc);
+    if (rc != SOCP_OK) return bail(ctx, rc);
+    with_model(model_id, [&](auto mo) { launch_traj<decltype(mo)::value>(ctx, B, S, in, d_Xf, tol, d_ns); });
+    if ((rc = last_launch(ctx)) != SOCP_OK || (rc = fetch_out(ctx, Xf, d_Xf, (size_t)B * N, mem)) != SOCP_OK ||
+        (rc = fetch_out(ctx, nsteps, d_ns, (size_t)B * 2, mem)) != SOCP_OK)
+        return bail(ctx, rc);
+    return finish(ctx, mem);
 }
 
 extern "C" {
 
 // ---- static facts ---------------------------------------------------------------------------
-int socp_model_dim(int id) { return (id >= 0 && id < SOCP_NUM_MODELS) ? kDim[id] : SOCP_ERR_ARG; }
-int socp_model_nparams(int id) { return (id >= 0 && id < SOCP_NUM_MODELS) ? kNP[id] : SOCP_ERR_ARG; }
-int socp_model_default_steps(int id) { return (id >= 0 && id < SOCP_NUM_MODELS) ? kSteps[id] : SOCP_ERR_ARG; }
+int socp_model_dim(int id) { return valid_model(id) ? model_facts(id).dim : SOCP_ERR_ARG; }
+int socp_model_nparams(int id) { return valid_model(id) ? model_facts(id).np : SOCP_ERR_ARG; }
+int socp_model_default_steps(int id) { return valid_model(id) ? model_facts(id).steps : SOCP_ERR_ARG; }
 int socp_model_default_params(int id, double *out) {
-    if (id < 0 || id >= SOCP_NUM_MODELS || !out) return SOCP_ERR_ARG;
-    for (int i = 0; i < kNP[id]; ++i) out[i] = kDefaults[id][i];
+    if (!valid_model(id) || !out) return SOCP_ERR_ARG;
+    std::copy_n(kDefaults[id], model_facts(id).np, out);
     return SOCP_OK;
 }
 int socp_num_param(const socp_shape *s) {
-    if (!s || s->model_id < 0 || s->model_id >= SOCP_NUM_MODELS || s->num_multi < 1 ||
-        s->num_multi >= SOCP_MAX_NODES)
+    if (!s || !valid_model(s->model_id) || s->num_multi < 1 || s->num_multi >= SOCP_MAX_NODES)
         return SOCP_ERR_ARG;
     int nfree = 0;
     for (int j = 0; j <= s->num_multi; ++j)
         if (s->mode_t[j] == SOCP_FREE) ++nfree;
-    return 2 * kDim[s->model_id] * s->num_multi + nfree;
+    return 2 * model_facts(s->model_id).dim * s->num_multi + nfree;
 }
 
 // ---- context --------------------------------------------------------------------------------
@@ -347,74 +408,20 @@ int socp_set_obstacles(socp_ctx *ctx, int n, const double *type, const double *p
 int socp_traj_batch(socp_ctx *ctx, int model_id, int step_nbr, long B, const double *mparams,
                     const double *sw, const double *t0, const double *tf, const double *X0,
                     double *Xf, int mem) {
-    if (!ctx) return SOCP_ERR_ARG;
-    if (model_id < 0 || model_id >= SOCP_NUM_MODELS || B < 0 || !mparams || !t0 || !tf || !X0 || !Xf)
-        return fail(ctx, SOCP_ERR_ARG, "socp_traj_batch: bad arguments");
-    if (B == 0) return SOCP_OK;
-    CUDA_TRY(ctx, cudaSetDevice(ctx->device));
-    const int N = 2 * kDim[model_id], np = kNP[model_id];
-    const int S = step_nbr > 0 ? step_nbr : kSteps[model_id];
-    int rc = SOCP_OK;
-    const double *d_mp = stage_in(ctx, SLOT_MPARAMS, mparams, (size_t)B * np, mem, &rc);
-    const double *d_sw = stage_in(ctx, SLOT_SW, sw, (size_t)B * 2, mem, &rc);
-    const double *d_t0 = stage_in(ctx, SLOT_T0, t0, (size_t)B, mem, &rc);
-    const double *d_tf = stage_in(ctx, SLOT_TF, tf, (size_t)B, mem, &rc);
-    const double *d_X0 = stage_in(ctx, SLOT_X0, X0, (size_t)B * N, mem, &rc);
-    double *d_Xf = stage_out(ctx, SLOT_XF, Xf, (size_t)B * N, mem, &rc);
-    if (rc != SOCP_OK) return rc;
-    switch (model_id) {
-    case SOCP_GODDARD: launch_traj<GODDARD>(ctx, B, S, d_mp, d_sw, d_t0, d_tf, d_X0, d_Xf); break;
-    case SOCP_DOUBLE_INTEGRATOR: launch_traj<DOUBLE_INTEGRATOR>(ctx, B, S, d_mp, d_sw, d_t0, d_tf, d_X0, d_Xf); break;
-    case SOCP_COVID19: launch_traj<COVID19>(ctx, B, S, d_mp, d_sw, d_t0, d_tf, d_X0, d_Xf); break;
-    case SOCP_VTOL_UAV: launch_traj<VTOL_UAV>(ctx, B, S, d_mp, d_sw, d_t0, d_tf, d_X0, d_Xf); break;
-    case SOCP_INTERCEPTOR: launch_traj<INTERCEPTOR>(ctx, B, S, d_mp, d_sw, d_t0, d_tf, d_X0, d_Xf); break;
-    }
-    CUDA_TRY(ctx, cudaGetLastError());
-    if ((rc = fetch_out(ctx, Xf, d_Xf, (size_t)B * N, mem)) != SOCP_OK) return rc;
-    if (mem == SOCP_HOST) CUDA_TRY(ctx, cudaStreamSynchronize(ctx->stream));
-    return SOCP_OK;
+    return traj_batch(ctx, "socp_traj_batch", model_id, step_nbr, B, mparams, sw, t0, tf, X0, 0., Xf, nullptr, mem);
 }
 
 int socp_traj_adaptive_batch(socp_ctx *ctx, int model_id, int step_nbr, long B, const double *mparams,
                              const double *sw, const double *t0, const double *tf, const double *X0,
                              double tol, double *Xf, int *nsteps, int mem) {
-    if (!ctx) return SOCP_ERR_ARG;
-    if (model_id < 0 || model_id >= SOCP_NUM_MODELS || B < 0 || !mparams || !t0 || !tf || !X0 || !Xf || !(tol > 0.))
-        return fail(ctx, SOCP_ERR_ARG, "socp_traj_adaptive_batch: bad arguments");
-    if (B == 0) return SOCP_OK;
-    CUDA_TRY(ctx, cudaSetDevice(ctx->device));
-    const int N = 2 * kDim[model_id], np = kNP[model_id];
-    const int S = step_nbr > 0 ? step_nbr : kSteps[model_id];
-    int rc = SOCP_OK;
-    const double *d_mp = stage_in(ctx, SLOT_MPARAMS, mparams, (size_t)B * np, mem, &rc);
-    const double *d_sw = stage_in(ctx, SLOT_SW, sw, (size_t)B * 2, mem, &rc);
-    const double *d_t0 = stage_in(ctx, SLOT_T0, t0, (size_t)B, mem, &rc);
-    const double *d_tf = stage_in(ctx, SLOT_TF, tf, (size_t)B, mem, &rc);
-    const double *d_X0 = stage_in(ctx, SLOT_X0, X0, (size_t)B * N, mem, &rc);
-    double *d_Xf = stage_out(ctx, SLOT_XF, Xf, (size_t)B * N, mem, &rc);
-    int *d_ns = stage_out(ctx, SLOT_INFO, nsteps, (size_t)B * 2, mem, &rc);
-    if (rc != SOCP_OK) return rc;
-    switch (model_id) {
-    case SOCP_GODDARD: launch_traj<GODDARD>(ctx, B, S, d_mp, d_sw, d_t0, d_tf, d_X0, d_Xf, tol, d_ns); break;
-    case SOCP_DOUBLE_INTEGRATOR: launch_traj<DOUBLE_INTEGRATOR>(ctx, B, S, d_mp, d_sw, d_t0, d_tf, d_X0, d_Xf, tol, d_ns); break;
-    case SOCP_COVID19: launch_traj<COVID19>(ctx, B, S, d_mp, d_sw, d_t0, d_tf, d_X0, d_Xf, tol, d_ns); break;
-    case SOCP_VTOL_UAV: launch_traj<VTOL_UAV>(ctx, B, S, d_mp, d_sw, d_t0, d_tf, d_X0, d_Xf, tol, d_ns); break;
-    case SOCP_INTERCEPTOR: launch_traj<INTERCEPTOR>(ctx, B, S, d_mp, d_sw, d_t0, d_tf, d_X0, d_Xf, tol, d_ns); break;
-    }
-    CUDA_TRY(ctx, cudaGetLastError());
-    if ((rc = fetch_out(ctx, Xf, d_Xf, (size_t)B * N, mem)) != SOCP_OK) return rc;
-    if ((rc = fetch_out(ctx, nsteps, d_ns, (size_t)B * 2, mem)) != SOCP_OK) return rc;
-    if (mem == SOCP_HOST) CUDA_TRY(ctx, cudaStreamSynchronize(ctx->stream));
-    return SOCP_OK;
+    if (!(tol > 0.)) return fail(ctx, SOCP_ERR_ARG, "socp_traj_adaptive_batch: bad arguments");
+    return traj_batch(ctx, "socp_traj_adaptive_batch", model_id, step_nbr, B, mparams, sw, t0, tf, X0, tol, Xf, nsteps, mem);
 }
 
-int socp_trace_width(int id) {
-    static const int nctrl[SOCP_NUM_MODELS] = {3, 3, 1, 3, 2};
-    return (id >= 0 && id < SOCP_NUM_MODELS) ? 2 * kDim[id] + nctrl[id] + 3 : SOCP_ERR_ARG;
-}
+int socp_trace_width(int id) { return valid_model(id) ? model_facts(id).trace_width : SOCP_ERR_ARG; }
 int socp_trace_max_rows(int id, int step_nbr) {
-    if (id < 0 || id >= SOCP_NUM_MODELS) return SOCP_ERR_ARG;
-    const int S = step_nbr > 0 ? step_nbr : kSteps[id];
+    if (!valid_model(id)) return SOCP_ERR_ARG;
+    const int S = step_nbr > 0 ? step_nbr : model_facts(id).steps;
     return (S + 1) * (id == SOCP_INTERCEPTOR ? 2 : 1);
 }
 
@@ -422,70 +429,56 @@ int socp_trace_batch(socp_ctx *ctx, int model_id, int step_nbr, long B, const do
                      const double *sw, const double *t0, const double *tf, const double *X0,
                      double *rows, int *nrows, double *Xf, int mem) {
     if (!ctx) return SOCP_ERR_ARG;
-    if (model_id < 0 || model_id >= SOCP_NUM_MODELS || B < 0 || !mparams || !t0 || !tf || !X0 || !rows || !nrows)
+    if (!valid_model(model_id) || B < 0 || !mparams || !t0 || !tf || !X0 || !rows || !nrows)
         return fail(ctx, SOCP_ERR_ARG, "socp_trace_batch: bad arguments");
     if (B == 0) return SOCP_OK;
     CUDA_TRY(ctx, cudaSetDevice(ctx->device));
-    const int N = 2 * kDim[model_id], np = kNP[model_id];
-    const int S = step_nbr > 0 ? step_nbr : kSteps[model_id];
-    const int W = socp_trace_width(model_id), R = socp_trace_max_rows(model_id, S);
+    const ModelFacts m = model_facts(model_id);
+    const int N = 2 * m.dim, S = step_nbr > 0 ? step_nbr : m.steps;
+    const int W = m.trace_width, R = socp_trace_max_rows(model_id, S);
     int rc = SOCP_OK;
-    const double *d_mp = stage_in(ctx, SLOT_MPARAMS, mparams, (size_t)B * np, mem, &rc);
-    const double *d_sw = stage_in(ctx, SLOT_SW, sw, (size_t)B * 2, mem, &rc);
-    const double *d_t0 = stage_in(ctx, SLOT_T0, t0, (size_t)B, mem, &rc);
-    const double *d_tf = stage_in(ctx, SLOT_TF, tf, (size_t)B, mem, &rc);
-    const double *d_X0 = stage_in(ctx, SLOT_X0, X0, (size_t)B * N, mem, &rc);
+    const TrajIn in = stage_traj(ctx, B, m.np, N, mparams, sw, t0, tf, X0, mem, &rc);
     double *d_rows = stage_out(ctx, SLOT_AUX0, rows, (size_t)B * R * W, mem, &rc);
     int *d_nr = stage_out(ctx, SLOT_INFO, nrows, (size_t)B, mem, &rc);
     double *d_Xf = stage_out(ctx, SLOT_XF, Xf, (size_t)B * N, mem, &rc);
-    if (rc != SOCP_OK) return rc;
-    switch (model_id) {
-    case SOCP_GODDARD: launch_trace<GODDARD>(ctx, B, S, R, d_mp, d_sw, d_t0, d_tf, d_X0, d_rows, d_nr, d_Xf); break;
-    case SOCP_DOUBLE_INTEGRATOR: launch_trace<DOUBLE_INTEGRATOR>(ctx, B, S, R, d_mp, d_sw, d_t0, d_tf, d_X0, d_rows, d_nr, d_Xf); break;
-    case SOCP_COVID19: launch_trace<COVID19>(ctx, B, S, R, d_mp, d_sw, d_t0, d_tf, d_X0, d_rows, d_nr, d_Xf); break;
-    case SOCP_VTOL_UAV: launch_trace<VTOL_UAV>(ctx, B, S, R, d_mp, d_sw, d_t0, d_tf, d_X0, d_rows, d_nr, d_Xf); break;
-    case SOCP_INTERCEPTOR: launch_trace<INTERCEPTOR>(ctx, B, S, R, d_mp, d_sw, d_t0, d_tf, d_X0, d_rows, d_nr, d_Xf); break;
-    }
-    CUDA_TRY(ctx, cudaGetLastError());
-    if ((rc = fetch_out(ctx, rows, d_rows, (size_t)B * R * W, mem)) != SOCP_OK) return rc;
-    if ((rc = fetch_out(ctx, nrows, d_nr, (size_t)B, mem)) != SOCP_OK) return rc;
-    if ((rc = fetch_out(ctx, Xf, d_Xf, (size_t)B * N, mem)) != SOCP_OK) return rc;
-    if (mem == SOCP_HOST) CUDA_TRY(ctx, cudaStreamSynchronize(ctx->stream));
-    return SOCP_OK;
+    if (rc != SOCP_OK) return bail(ctx, rc);
+    with_model(model_id, [&](auto mo) {
+        trace_kernel<decltype(mo)::value><<<(unsigned)((B + 63) / 64), 64, 0, ctx->stream>>>(
+            B, S, R, in.mp, in.sw, in.t0, in.tf, in.X0, d_rows, d_nr, d_Xf);
+    });
+    ctx->launches += 1;
+    if ((rc = last_launch(ctx)) != SOCP_OK || (rc = fetch_out(ctx, rows, d_rows, (size_t)B * R * W, mem)) != SOCP_OK ||
+        (rc = fetch_out(ctx, nrows, d_nr, (size_t)B, mem)) != SOCP_OK || (rc = fetch_out(ctx, Xf, d_Xf, (size_t)B * N, mem)) != SOCP_OK)
+        return bail(ctx, rc);
+    return finish(ctx, mem);
 }
 
 int socp_point_batch(socp_ctx *ctx, int model_id, long B, const double *mparams, const double *sw,
                      const int *chart_stage, const double *t, const double *X, double *rhs,
                      double *control, double *H, int mem) {
     if (!ctx) return SOCP_ERR_ARG;
-    if (model_id < 0 || model_id >= SOCP_NUM_MODELS || B < 0 || !mparams || !t || !X)
+    if (!valid_model(model_id) || B < 0 || !mparams || !t || !X)
         return fail(ctx, SOCP_ERR_ARG, "socp_point_batch: bad arguments");
     if (B == 0) return SOCP_OK;
     CUDA_TRY(ctx, cudaSetDevice(ctx->device));
-    const int N = 2 * kDim[model_id], np = kNP[model_id];
+    const ModelFacts m = model_facts(model_id);
+    const int N = 2 * m.dim;
     int rc = SOCP_OK;
-    const double *d_mp = stage_in(ctx, SLOT_MPARAMS, mparams, (size_t)B * np, mem, &rc);
-    const double *d_sw = stage_in(ctx, SLOT_SW, sw, (size_t)B * 2, mem, &rc);
+    const TrajIn in = stage_traj(ctx, B, m.np, N, mparams, sw, t, nullptr, X, mem, &rc);
     const int *d_cs = stage_in(ctx, SLOT_INFO, chart_stage, (size_t)B * 2, mem, &rc);
-    const double *d_t = stage_in(ctx, SLOT_T0, t, (size_t)B, mem, &rc);
-    const double *d_X = stage_in(ctx, SLOT_X0, X, (size_t)B * N, mem, &rc);
     double *d_rhs = stage_out(ctx, SLOT_AUX0, rhs, (size_t)B * N, mem, &rc);
     double *d_ctl = stage_out(ctx, SLOT_AUX1, control, (size_t)B * 4, mem, &rc);
     double *d_H = stage_out(ctx, SLOT_AUX2, H, (size_t)B, mem, &rc);
-    if (rc != SOCP_OK) return rc;
-    switch (model_id) {
-    case SOCP_GODDARD: launch_point<GODDARD>(ctx, B, d_mp, d_sw, d_cs, d_t, d_X, d_rhs, d_ctl, d_H); break;
-    case SOCP_DOUBLE_INTEGRATOR: launch_point<DOUBLE_INTEGRATOR>(ctx, B, d_mp, d_sw, d_cs, d_t, d_X, d_rhs, d_ctl, d_H); break;
-    case SOCP_COVID19: launch_point<COVID19>(ctx, B, d_mp, d_sw, d_cs, d_t, d_X, d_rhs, d_ctl, d_H); break;
-    case SOCP_VTOL_UAV: launch_point<VTOL_UAV>(ctx, B, d_mp, d_sw, d_cs, d_t, d_X, d_rhs, d_ctl, d_H); break;
-    case SOCP_INTERCEPTOR: launch_point<INTERCEPTOR>(ctx, B, d_mp, d_sw, d_cs, d_t, d_X, d_rhs, d_ctl, d_H); break;
-    }
-    CUDA_TRY(ctx, cudaGetLastError());
-    if ((rc = fetch_out(ctx, rhs, d_rhs, (size_t)B * N, mem)) != SOCP_OK) return rc;
-    if ((rc = fetch_out(ctx, control, d_ctl, (size_t)B * 4, mem)) != SOCP_OK) return rc;
-    if ((rc = fetch_out(ctx, H, d_H, (size_t)B, mem)) != SOCP_OK) return rc;
-    if (mem == SOCP_HOST) CUDA_TRY(ctx, cudaStreamSynchronize(ctx->stream));
-    return SOCP_OK;
+    if (rc != SOCP_OK) return bail(ctx, rc);
+    with_model(model_id, [&](auto mo) {
+        point_kernel<decltype(mo)::value><<<(unsigned)((B + 127) / 128), 128, 0, ctx->stream>>>(
+            B, in.mp, in.sw, d_cs, in.t0, in.X0, d_rhs, d_ctl, d_H);
+    });
+    ctx->launches += 1;
+    if ((rc = last_launch(ctx)) != SOCP_OK || (rc = fetch_out(ctx, rhs, d_rhs, (size_t)B * N, mem)) != SOCP_OK ||
+        (rc = fetch_out(ctx, control, d_ctl, (size_t)B * 4, mem)) != SOCP_OK || (rc = fetch_out(ctx, H, d_H, (size_t)B, mem)) != SOCP_OK)
+        return bail(ctx, rc);
+    return finish(ctx, mem);
 }
 
 // ---- FP64 peak probe ------------------------------------------------------------------------

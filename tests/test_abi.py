@@ -34,6 +34,14 @@ def test_static_facts():
     for m in range(5):
         assert list(sb.default_params(m)) == pytest.approx(S.DEFAULTS[m])
         assert sb.PARAM_NAMES[m] == S.PARAMS[m]
+        assert sb.model_nparams(m) == len(S.DEFAULTS[m])
+    # the caller's trace buffer is sized from these: a row is model::Trace (t, X, controls, H, extra), 2 dim + nctrl + 3
+    from socp_b200 import _lib
+    L = _lib.lib()
+    assert [L.socp_trace_width(m) for m in range(5)] == [20, 18, 12, 18, 17]
+    # one integration of S steps gives S + 1 rows; the interceptor's trace has two stages
+    assert L.socp_trace_max_rows(sb.INTERCEPTOR, 10) == 22
+    assert L.socp_trace_max_rows(sb.GODDARD, 10) == 11
     mode_t, mode_X = sb.default_modes(sb.GODDARD, 6, sb.FREE, S.GODDARD_MODE_XF)
     assert sb.num_param(sb.make_shape(sb.GODDARD, 6, mode_t, mode_X)) == 85
 
