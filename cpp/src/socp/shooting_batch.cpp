@@ -1,5 +1,6 @@
 // cpp/src/socp/shooting_batch.cpp -- see shooting_batch.hpp.  Host bookkeeping only; the numerical
-// work is socp_traj_batch / socp_solve_batch / socp_continuation_*_batch (include/socp_b200.h).
+// work is socp_traj_batch / socp_solve_batch / socp_continuation_*_batch / socp_move_batch /
+// socp_solution_batch (include/socp_b200.h).
 #include <cstdlib>
 #include <cstring>
 #include <functional>
@@ -63,13 +64,11 @@ shooting_batch::shooting_batch(model & model, int numMulti, long batch, int numD
 		for (int g = 0; g < data->numDevice; g++) data->devices.push_back(data->numDevice == 1 && dev ? atoi(dev) : g);
 	}
 	data->dim = model.GetDim();
-	data->numMulti = numMulti;
 	data->xtol = 1e-8;						// shooting.cpp:95-101
 	data->maxfev = 10000;
 	data->stepMin = 1e-12;
 	memset(&data->shape, 0, sizeof data->shape);
 	data->shape.model_id = model.DeviceModelId();
-	data->shape.num_multi = numMulti;
 	data->shape.step_nbr = model.DeviceSteps();
 	data->shape.integrator = model.deviceAdaptive ? SOCP_DOPRI5 : SOCP_RK4;
 	data->shape.ode_tol = model.odeIntTol;
@@ -77,9 +76,7 @@ shooting_batch::shooting_batch(model & model, int numMulti, long batch, int numD
 	data->np = (int)block.size();
 	data->mparams.resize((size_t)batch * data->np);
 	for (long k = 0; k < batch; k++) std::copy(block.begin(), block.end(), data->mparams.begin() + k * data->np);
-	const size_t nodes = numMulti + 1;
-	data->time.assign(batch * nodes, 0); data->timed = data->time; data->time_prec = data->time;
-	data->X.assign(batch * nodes * data->dim, 0); data->Xd = data->X; data->X_prec = data->X;
+	Resize(numMulti);
 	data->info.assign(batch, 0); data->nfev.assign(batch, 0); data->calls.assign(batch, 0);
 	data->fnorm.assign(batch, 0);
 	std::vector<int> fixed(data->dim, model::FIXED);
@@ -87,6 +84,18 @@ shooting_batch::shooting_batch(model & model, int numMulti, long batch, int numD
 }
 
 shooting_batch::~shooting_batch() { delete data; }
+
+void shooting_batch::Resize(int numMulti) {
+	if (numMulti < 1 || numMulti >= SOCP_MAX_NODES) {
+		std::cerr << std::endl << "ERROR : shooting_batch needs 1 <= numMulti < " << SOCP_MAX_NODES << std::endl;
+		exit(1);
+	}
+	data->numMulti = numMulti;
+	data->shape.num_multi = numMulti;
+	const size_t nodes = numMulti + 1;
+	data->time.assign(data->B * nodes, 0); data->timed = data->time; data->time_prec = data->time;
+	data->X.assign(data->B * nodes * data->dim, 0); data->Xd = data->X; data->X_prec = data->X;
+}
 
 long shooting_batch::GetBatch() const { return data->B; }
 int shooting_batch::GetNumDevice() const { return data->numDevice; }
@@ -174,6 +183,10 @@ void shooting_batch::InitShooting(long k, std::vector<real> const& vt, std::vect
 		if (data->shape.mode_t[j] == model::FREE) data->param[k * P + q++] = vt[j];
 }
 
+void shooting_batch::InitShooting(std::vector< std::vector<real> > const& vt, std::vector< std::vector<model::mstate> > const& vX) {
+	for (long k = 0; k < data->B; k++) InitShooting(k, vt[k], vX[k]);
+}
+
 void shooting_batch::SetDesiredState(long k, real const& ti, model::mstate const& Xi, real const& tf, model::mstate const& Xf) {
 	const int M = data->numMulti, n = data->dim, nodes = M + 1;
 	data->timed[k * nodes] = ti;
@@ -235,7 +248,9 @@ long shooting_batch::SolveOCP(real const& continuationStep) {
 	for (long k = 0; k < B; k++) {
 		data->calls[k] = calls[2 * k];
 		data->nfev[k] = calls[2 * k + 1];
-		if (data->info[k] == 1) {				// the homotopy arrived: desired data become the previous data
+		if (data->info[k] == 1) {				// the homotopy arrived: desired data become the current and previous data
+			std::copy(data->timed.begin() + k * nodes, data->timed.begin() + (k + 1) * nodes, data->time.begin() + k * nodes);
+			std::copy(data->Xd.begin() + k * nodes * n, data->Xd.begin() + (k + 1) * nodes * n, data->X.begin() + k * nodes * n);
 			std::copy(data->timed.begin() + k * nodes, data->timed.begin() + (k + 1) * nodes, data->time_prec.begin() + k * nodes);
 			std::copy(data->Xd.begin() + k * nodes * n, data->Xd.begin() + (k + 1) * nodes * n, data->X_prec.begin() + k * nodes * n);
 		}
@@ -277,3 +292,38 @@ void shooting_batch::GetParameters(long k, std::vector<real> & paramVector) cons
 }
 
 real shooting_batch::GetParameters(long k, int i) const { return data->param[k * data->numParam + i]; }
+
+void shooting_batch::Move(std::vector<real> const& tf, std::vector<model::mstate> & Xf) const {
+	const long B = data->B;
+	const int P = data->numParam, np = data->np, N = 2 * data->dim;
+	const size_t nodes = data->numMulti + 1;
+	std::vector<real> Xq((size_t)B * N);
+	const data_struct *d = data;
+	data->for_each_block([&, d](socp_ctx *ctx, long lo, long hi) {
+		if (socp_move_batch(ctx, &d->shape, hi - lo, d->mparams.data() + lo * np, d->time.data() + lo * nodes,
+		                    d->param.data() + lo * P, 1, tf.data() + lo, Xq.data() + lo * N, SOCP_HOST) != SOCP_OK)
+			fail(ctx, "socp_move_batch");
+	});
+	Xf.resize(B);
+	for (long k = 0; k < B; k++) Xf[k].assign(Xq.begin() + k * N, Xq.begin() + (k + 1) * N);
+}
+
+void shooting_batch::GetSolution(std::vector< std::vector<real> > & vt, std::vector< std::vector<model::mstate> > & vX) const {
+	const long B = data->B;
+	const int P = data->numParam, np = data->np, N = 2 * data->dim, M = data->numMulti;
+	const size_t nodes = M + 1;
+	std::vector<real> t((size_t)B * nodes), X((size_t)B * nodes * N);
+	const data_struct *d = data;
+	data->for_each_block([&, d](socp_ctx *ctx, long lo, long hi) {
+		if (socp_solution_batch(ctx, &d->shape, hi - lo, d->mparams.data() + lo * np, d->time.data() + lo * nodes,
+		                        d->param.data() + lo * P, t.data() + lo * nodes, X.data() + lo * nodes * N, SOCP_HOST) != SOCP_OK)
+			fail(ctx, "socp_solution_batch");
+	});
+	vt.resize(B);
+	vX.resize(B);
+	for (long k = 0; k < B; k++) {
+		vt[k].assign(t.begin() + k * nodes, t.begin() + (k + 1) * nodes);
+		vX[k].resize(nodes);
+		for (size_t i = 0; i < nodes; i++) vX[k][i].assign(X.begin() + (k * nodes + i) * N, X.begin() + (k * nodes + i + 1) * N);
+	}
+}

@@ -1,8 +1,9 @@
 // cpp/src/socp/shooting_batch.hpp -- the batch driver the reference does not have: B independent
 // shooting problems that share one model type and one mode layout, solved together on the GPU.
 // Same vocabulary and semantics as `shooting` (shooting.hpp), with a leading problem index:
-// SetMode / InitShooting / SetDesiredState / SolveOCP / GetParameters / GetSolution.  One call of
-// SolveOCP is one socp_solve_batch (or one batched continuation) over all B problems.
+// Resize / SetMode / InitShooting / SetDesiredState / SolveOCP / GetParameters, and Move / GetSolution to
+// sample the solutions and re-mesh them.  One call of SolveOCP is one socp_solve_batch (or one batched
+// continuation) over all B problems; one Move or GetSolution is one socp_move_batch / socp_solution_batch.
 #include <vector>
 
 #include "model.hpp"
@@ -23,6 +24,10 @@ public:
 	int GetNumDevice() const;
 	int GetNumParam() const;
 
+	/// shooting::Resize(numMulti) for every problem: the node arrays take the new size (their contents are
+	/// reset) and, as in the reference, SetMode must follow before InitShooting
+	void Resize(int numMulti);
+
 	void SetMode(int const& mode_tf, std::vector<int> const& mode_Xf);
 	void SetMode(std::vector<int> const& mode_t, std::vector< std::vector<int> > const& mode_X);
 
@@ -37,6 +42,8 @@ public:
 	                  std::vector<real> const& tf, std::vector<model::mstate> const& Xf);
 	/// shooting::InitShooting(vt, vX) for problem k
 	void InitShooting(long k, std::vector<real> const& vt, std::vector<model::mstate> const& vX);
+	/// shooting::InitShooting(vt, vX) for every problem: vt[k] has M+1 node times, vX[k] M+1 node states
+	void InitShooting(std::vector< std::vector<real> > const& vt, std::vector< std::vector<model::mstate> > const& vX);
 	void SetDesiredState(long k, real const& ti, model::mstate const& Xi, real const& tf, model::mstate const& Xf);
 	void SetDesiredState(long k, std::vector<real> const& vt, std::vector<model::mstate> const& vX);
 
@@ -55,6 +62,12 @@ public:
 	real GetResidualNorm(long k) const;
 	void GetParameters(long k, std::vector<real> & paramVector) const;
 	real GetParameters(long k, int i) const;
+
+	/// shooting::Move(tf) for every problem: Xf[k] = state of solution k at tf[k] (a time outside [t0, t_end] gives
+	/// the state at t_end)
+	void Move(std::vector<real> const& tf, std::vector<model::mstate> & Xf) const;
+	/// shooting::GetSolution for every problem: vt[k] = the M+1 node times, vX[k] = the node states, vX[k][M] = Move(t_end)
+	void GetSolution(std::vector< std::vector<real> > & vt, std::vector< std::vector<model::mstate> > & vX) const;
 
 private:
 	model & myModel;

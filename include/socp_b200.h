@@ -15,7 +15,7 @@
  * or SOCP_DEVICE (device pointers on the context's device; results are ordered on the context
  * stream: socp_sync() before reading them from another stream).  The batched solves and continuations
  * block the calling host thread intermittently: the round loop reads device-side work counters every
- * few rounds to know when the last problem has retired; the trajectory / residual / Jacobian calls only enqueue.  There is no CPU fallback: without a CUDA device
+ * few rounds to know when the last problem has retired; the trajectory / residual / Jacobian / Move / GetSolution calls only enqueue.  There is no CPU fallback: without a CUDA device
  * socp_create fails.
  *
  * Data layouts (all double unless noted, row-major, one problem after another):
@@ -208,6 +208,22 @@ int socp_continuation_boundary_batch(socp_ctx *ctx, const socp_shape *shape, lon
                                      const double *Xb_prec, const double *time_des,
                                      const double *Xb_des, double *x, double xtol, int maxfev,
                                      double step, double step_min, int *info, int *calls, int mem);
+
+/* Sampling a solution (the unknowns x [B][P] of a solve, with the time [B][M+1] and mparams it was solved with).
+ * shooting::Move(tf) (shooting.cpp:383-437) of B solutions x at Q query times each: tq [B][Q], Xq [B][Q][2dim].
+ * The time line is ComputeTimeLine's (FREE times from x, CONTINUOUS nodes interpolated), which also sets goddard's
+ * switching times; the state is the integration of the segment that holds the target from its node state:
+ * seg = 0; while (tl[seg+1] < target) ++seg -- so a query at node time tl[j+1] returns the end of segment j, not
+ * node j+1.  A query outside [t0, t_end] (NaN included) is answered at t_end, as in the reference.  A Move is bit
+ * for bit the socp_traj_batch (or, with SOCP_DOPRI5, socp_traj_adaptive_batch) of the same segment start, node
+ * state, target and switching times.  Q == 0 or B == 0: nothing is done. */
+int socp_move_batch(socp_ctx *ctx, const socp_shape *shape, long B, const double *mparams, const double *time,
+                    const double *x, int Q, const double *tq, double *Xq, int mem);
+/* shooting::GetSolution (shooting.cpp:481-488, UpdateSolution :1462-1508): vt [B][M+1] node times of the
+ * solution, vX [B][M+1][2dim] node states (vX[i] = node i of x for i < M, vX[M] = Move(t_end)).  The result is the
+ * node data of a re-mesh: Move at the new node times, then InitShooting(vt, vX). */
+int socp_solution_batch(socp_ctx *ctx, const socp_shape *shape, long B, const double *mparams, const double *time,
+                        const double *x, double *vt, double *vX, int mem);
 
 /* FP64 FMA peak of the device measured with a register-resident DFMA chain (GFLOP/s). */
 int socp_measure_fp64_peak(socp_ctx *ctx, double *gflops, double *sm_clock_mhz);

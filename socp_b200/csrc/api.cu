@@ -16,6 +16,7 @@
 #include "models.cuh"
 #include "integrate.cuh"
 #include "solver.cuh"
+#include "move.cuh"
 
 using namespace socp;
 

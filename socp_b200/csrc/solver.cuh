@@ -186,9 +186,10 @@ SOCP_DEV void timeline_all(const SolverDev &D, const double *time_b, XF xfree, d
         }
     }
 }
-// the two node times of segment s without materialising the whole line
-template <class XF>
-SOCP_DEV void timeline_pair(const SolverDev &D, const double *time_b, XF xfree, int s, double &t1, double &t2, double *sw) {
+// the two node times of segment s without materialising the whole line.  SH is any shape with M and mode_t[M + 1]:
+// SolverDev for the solver kernels, MoveShape for the move kernel (move.cuh).
+template <class SH, class XF>
+SOCP_DEV void timeline_pair(const SH &D, const double *time_b, XF xfree, int s, double &t1, double &t2, double *sw) {
     int k = 0, cur = 0, nsw = 0;
     double tcur = 0;
     t1 = t2 = 0;

@@ -72,6 +72,26 @@ def num_param(shape):
     return _lib.lib().socp_num_param(ctypes.byref(shape))
 
 
+def unknowns_from_nodes(shape, vt, vX):
+    """shooting::InitShooting(vt, vX) (shooting.cpp:88-114) for B problems of one shape: the unknowns x[B][P] (the
+    M node blocks vX[:, :M], then the FREE node times in node order) and the boundary / waypoint states
+    Xb = vX[..., :dim].  vt is [B][M+1], vX [B][M+1][2dim]; numpy arrays give numpy results, torch tensors give
+    tensors on the same device (no copy through the host).  The node times of the new problem are vt itself."""
+    M, dim = shape.num_multi, model_dim(shape.model_id)
+    N = 2 * dim
+    free = [j for j in range(M + 1) if shape.mode_t[j] == FREE]
+    if tuple(vX.shape[1:]) != (M + 1, N) or tuple(vt.shape[1:]) != (M + 1,) or vt.shape[0] != vX.shape[0]:
+        raise ValueError("vt must be [B][%d] and vX [B][%d][%d]" % (M + 1, M + 1, N))
+    B = vX.shape[0]
+    if _is_torch(vX):
+        import torch
+        x = torch.cat([vX[:, :M].reshape(B, M * N), vt[:, free]], dim=1)
+        return x, vX[..., :dim].contiguous()
+    vt, vX = np.asarray(vt, dtype=np.float64), np.asarray(vX, dtype=np.float64)
+    x = np.concatenate([vX[:, :M].reshape(B, M * N), vt[:, free]], axis=1)
+    return x, np.ascontiguousarray(vX[..., :dim])
+
+
 def _is_torch(a):
     return a is not None and type(a).__module__.startswith("torch")
 
@@ -333,6 +353,46 @@ class Engine:
                                              a.inp(Xb), a.out(x), float(xtol), int(maxfev), a.out(info, np.int32),
                                              a.out(nfev, np.int32), a.out(fnorm), mem))
         return dict(x=x, info=info, nfev=nfev, fnorm=fnorm)
+
+    def move_batch(self, shape, mparams, time, x, tq, out=None):
+        """shooting::Move(tf) of B solutions x at Q times each (socp_move_batch): tq [B][Q] (host arrays: a [Q]
+        vector is shared by every problem); returns Xq [B][Q][2dim].  A time outside [t0, t_end] gives the
+        state at t_end, as in the reference."""
+        mem, B, mparams = self._problem_args(shape, mparams, time, None, x)
+        N = 2 * model_dim(shape.model_id)
+        if mem == HOST:
+            tq = np.asarray(tq, dtype=np.float64)
+            tq = np.ascontiguousarray(np.broadcast_to(tq, (B, tq.shape[-1])) if tq.ndim == 1 else tq)
+            Q = tq.shape[1]
+            if out is None:
+                out = np.empty((B, Q, N))
+        else:
+            Q = tq.shape[1]
+            if out is None:
+                import torch
+                out = torch.empty((B, Q, N), dtype=torch.float64, device=x.device)
+        if tuple(tq.shape) != (B, Q):
+            raise ValueError("tq must be [B][Q]")
+        a = self._arg(mem)
+        self._check(self._L.socp_move_batch(self._h, ctypes.byref(shape), B, a.inp(mparams), a.inp(time), a.inp(x),
+                                            int(Q), a.inp(tq), a.out(out), mem))
+        return out
+
+    def solution_batch(self, shape, mparams, time, x):
+        """shooting::GetSolution for B solutions (socp_solution_batch): returns (vt [B][M+1], vX [B][M+1][2dim]),
+        vX[:, M] = Move(t_end).  Numpy arrays or torch CUDA tensors, like solve_batch."""
+        mem, B, mparams = self._problem_args(shape, mparams, time, None, x)
+        M, N = shape.num_multi, 2 * model_dim(shape.model_id)
+        if mem == HOST:
+            vt, vX = np.empty((B, M + 1)), np.empty((B, M + 1, N))
+        else:
+            import torch
+            vt = torch.empty((B, M + 1), dtype=torch.float64, device=x.device)
+            vX = torch.empty((B, M + 1, N), dtype=torch.float64, device=x.device)
+        a = self._arg(mem)
+        self._check(self._L.socp_solution_batch(self._h, ctypes.byref(shape), B, a.inp(mparams), a.inp(time), a.inp(x),
+                                                a.out(vt), a.out(vX), mem))
+        return vt, vX
 
     # -- analytic-Jacobian path (modelOrder == 1; the double integrator, as in the reference) -----
     def traj_var_batch(self, model_id, mparams, t0, X0, tf, step_nbr=0):
