@@ -132,20 +132,7 @@ model::mstate model::ModelInt(real const& t0, mstate const& X, real const& tf, i
 		if (socp_trace_batch(dc.ctx, dc.id, DeviceSteps(), 1, dc.mp.data(), dc.sw, &t0, &tf, Xin.data(), rows.data(), &nrows,
 		                     Xout.data(), SOCP_HOST) != SOCP_OK)
 			die("socp_trace_batch", dc.ctx);
-		// same text as model::Trace (model.hpp:446-462): default ostream precision, tab separated
-		std::stringstream ss;
-		const int nc = W - N - 3;
-		for (int r = 0; r < nrows; r++) {
-			const real *row = &rows[(size_t)r * W];
-			ss << row[0] << "\t";
-			for (int k = 0; k < N; k++) ss << row[1 + k] << "\t";
-			for (int k = 0; k < nc; k++) ss << row[1 + N + k] << "\t";
-			TraceTail(row[1 + N + nc], row[2 + N + nc], ss);
-		}
-		std::ofstream fileTrace;
-		fileTrace.open(strFileTrace.c_str(), std::ios::app);
-		fileTrace << ss.str();
-		fileTrace.close();
+		AppendTrace(rows.data(), &nrows, 1, R);
 	} else if (deviceAdaptive) {
 		if (socp_traj_adaptive_batch(dc.ctx, dc.id, DeviceSteps(), 1, dc.mp.data(), dc.sw, &t0, &tf, Xin.data(), odeIntTol,
 		                             Xout.data(), nullptr, SOCP_HOST) != SOCP_OK)
@@ -218,6 +205,24 @@ void model::SwitchingTimesUpdate(std::vector<real> const& switchingTimes) { devi
 
 // -------------------------------------------------------------------------------------------------
 void model::TraceTail(real H, real, std::ostream & file) const { file << H << std::endl; }
+
+void model::AppendTrace(const real *rows, const int *nrows, int nseg, int R) const {
+	// same text as model::Trace (model.hpp:446-462): default ostream precision, tab separated
+	const int N = 2 * dim, W = socp_trace_width(DeviceModelId()), nc = W - N - 3;
+	std::stringstream ss;
+	for (int s = 0; s < nseg; s++)
+		for (int r = 0; r < nrows[s]; r++) {
+			const real *row = rows + ((size_t)s * R + r) * W;
+			ss << row[0] << "\t";
+			for (int k = 0; k < N; k++) ss << row[1 + k] << "\t";
+			for (int k = 0; k < nc; k++) ss << row[1 + N + k] << "\t";
+			TraceTail(row[1 + N + nc], row[2 + N + nc], ss);
+		}
+	std::ofstream fileTrace;
+	fileTrace.open(strFileTrace.c_str(), std::ios::app);
+	fileTrace << ss.str();
+	fileTrace.close();
+}
 
 template <class S> static void trace_point(const model &m, real const& t, model::mstate const& X, S & file) {
 	model::mcontrol u = m.Control(t, X);

@@ -78,6 +78,10 @@ public:
 	/// end of a trace row: H, then whatever the model appends (goddard: switching function,
 	/// goddard.cpp:337; interceptor: chart id, interceptor.cpp:151); `extra` is the device's last column
 	virtual void TraceTail(real H, real extra, std::ostream & file) const;
+	/// trace rows in the layout of socp_trace_batch (rows [nseg][R][socp_trace_width], nrows [nseg]) appended to
+	/// strFileTrace as model::Trace writes them; ModelInt's trace branch, shooting::Trace and shooting_batch::Trace(k)
+	/// all write through it
+	void AppendTrace(const real *rows, const int *nrows, int nseg, int R) const;
 	static socp_ctx* Context();					///< engine context of the default device (device 0 or $SOCP_DEVICE)
 	/// engine context of CUDA device `device` (one context per device, created on first use; thread safe).
 	/// The obstacle table set through SetDeviceObstacles is replayed on every context created later.

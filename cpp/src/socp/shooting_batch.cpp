@@ -1,6 +1,6 @@
 // cpp/src/socp/shooting_batch.cpp -- see shooting_batch.hpp.  Host bookkeeping only; the numerical
 // work is socp_traj_batch / socp_solve_batch / socp_continuation_*_batch / socp_move_batch /
-// socp_solution_batch (include/socp_b200.h).
+// socp_solution_batch / socp_solution_trace_batch (include/socp_b200.h).
 #include <cstdlib>
 #include <cstring>
 #include <functional>
@@ -326,4 +326,32 @@ void shooting_batch::GetSolution(std::vector< std::vector<real> > & vt, std::vec
 		vX[k].resize(nodes);
 		for (size_t i = 0; i < nodes; i++) vX[k][i].assign(X.begin() + (k * nodes + i) * N, X.begin() + (k * nodes + i + 1) * N);
 	}
+}
+
+void shooting_batch::Trace(std::vector<real> & rows, std::vector<int> & nrows) const {
+	const long B = data->B;
+	const int P = data->numParam, np = data->np, M = data->numMulti;
+	const size_t nodes = M + 1;
+	const size_t per = (size_t)M * socp_trace_max_rows(data->shape.model_id, data->shape.step_nbr) * socp_trace_width(data->shape.model_id);
+	rows.resize(B * per);
+	nrows.resize((size_t)B * M);
+	const data_struct *d = data;
+	data->for_each_block([&, d](socp_ctx *ctx, long lo, long hi) {
+		if (socp_solution_trace_batch(ctx, &d->shape, hi - lo, d->mparams.data() + lo * np, d->time.data() + lo * nodes,
+		                              d->param.data() + lo * P, rows.data() + lo * per, nrows.data() + lo * M, SOCP_HOST) != SOCP_OK)
+			fail(ctx, "socp_solution_trace_batch");
+	});
+}
+
+void shooting_batch::Trace(long k) const {
+	const int P = data->numParam, np = data->np, M = data->numMulti;
+	const size_t nodes = M + 1;
+	const int R = socp_trace_max_rows(data->shape.model_id, data->shape.step_nbr);
+	std::vector<real> rows((size_t)M * R * socp_trace_width(data->shape.model_id));
+	std::vector<int> nrows(M);
+	socp_ctx *ctx = model::Context(data->devices[0]);
+	if (socp_solution_trace_batch(ctx, &data->shape, 1, data->mparams.data() + k * np, data->time.data() + k * nodes,
+	                              data->param.data() + k * P, rows.data(), nrows.data(), SOCP_HOST) != SOCP_OK)
+		fail(ctx, "socp_solution_trace_batch");
+	myModel.AppendTrace(rows.data(), nrows.data(), M, R);
 }

@@ -1,9 +1,10 @@
 // cpp/src/socp/shooting_batch.hpp -- the batch driver the reference does not have: B independent
 // shooting problems that share one model type and one mode layout, solved together on the GPU.
 // Same vocabulary and semantics as `shooting` (shooting.hpp), with a leading problem index:
-// Resize / SetMode / InitShooting / SetDesiredState / SolveOCP / GetParameters, and Move / GetSolution to
-// sample the solutions and re-mesh them.  One call of SolveOCP is one socp_solve_batch (or one batched
-// continuation) over all B problems; one Move or GetSolution is one socp_move_batch / socp_solution_batch.
+// Resize / SetMode / InitShooting / SetDesiredState / SolveOCP / GetParameters, Move / GetSolution to
+// sample the solutions and re-mesh them, and Trace.  One call of SolveOCP is one socp_solve_batch (or one batched
+// continuation) over all B problems; one Move, GetSolution or Trace is one socp_move_batch / socp_solution_batch /
+// socp_solution_trace_batch.
 #include <vector>
 
 #include "model.hpp"
@@ -68,6 +69,11 @@ public:
 	void Move(std::vector<real> const& tf, std::vector<model::mstate> & Xf) const;
 	/// shooting::GetSolution for every problem: vt[k] = the M+1 node times, vX[k] = the node states, vX[k][M] = Move(t_end)
 	void GetSolution(std::vector< std::vector<real> > & vt, std::vector< std::vector<model::mstate> > & vX) const;
+	/// shooting::Trace for every problem: every segment re-integrated with the observer on, in the layout of
+	/// socp_solution_trace_batch -- rows [B][M][R][W] (R = socp_trace_max_rows, W = socp_trace_width), nrows [B][M]
+	void Trace(std::vector<real> & rows, std::vector<int> & nrows) const;
+	/// shooting::Trace of problem k: its rows appended to the model's trace file, the text shooting::Trace writes
+	void Trace(long k) const;
 
 private:
 	model & myModel;

@@ -15,7 +15,7 @@
  * or SOCP_DEVICE (device pointers on the context's device; results are ordered on the context
  * stream: socp_sync() before reading them from another stream).  The batched solves and continuations
  * block the calling host thread intermittently: the round loop reads device-side work counters every
- * few rounds to know when the last problem has retired; the trajectory / residual / Jacobian / Move / GetSolution calls only enqueue.  There is no CPU fallback: without a CUDA device
+ * few rounds to know when the last problem has retired; the trajectory / residual / Jacobian / Move / GetSolution / Trace calls only enqueue.  There is no CPU fallback: without a CUDA device
  * socp_create fails.
  *
  * Data layouts (all double unless noted, row-major, one problem after another):
@@ -224,6 +224,17 @@ int socp_move_batch(socp_ctx *ctx, const socp_shape *shape, long B, const double
  * node data of a re-mesh: Move at the new node times, then InitShooting(vt, vX). */
 int socp_solution_batch(socp_ctx *ctx, const socp_shape *shape, long B, const double *mparams, const double *time,
                         const double *x, double *vt, double *vX, int mem);
+/* shooting::Trace (shooting.cpp:496-544): every segment of B solutions re-integrated with the observer on.
+ * rows [B][M][R][W] and nrows [B][M] (int): rows[b][j] holds the nrows[b][j] rows of segment j of problem b in the
+ * layout of socp_trace_batch (R = socp_trace_max_rows(model, step_nbr), W = socp_trace_width(model)); rows past
+ * nrows[b][j] are unspecified.  Segment j runs from node time tl[j] (ComputeTimeLine's, as for a Move) and node
+ * state j of x to tl[j+1], so it is bit for bit the socp_trace_batch of the same start, node state, end, switching
+ * times and step_nbr: S+1 rows, 2(S+1) for an interceptor segment that crosses the burn-out time.  The first row of
+ * segment j+1 repeats the node time tl[j+1] that ends segment j, as in the reference's trace file.  A SOCP_DOPRI5
+ * shape is traced with the fixed-step RK4 observer too (odeTools.cpp:103-123): the reference has no adaptive
+ * observer.  B == 0: nothing is done. */
+int socp_solution_trace_batch(socp_ctx *ctx, const socp_shape *shape, long B, const double *mparams, const double *time,
+                              const double *x, double *rows, int *nrows, int mem);
 
 /* FP64 FMA peak of the device measured with a register-resident DFMA chain (GFLOP/s). */
 int socp_measure_fp64_peak(socp_ctx *ctx, double *gflops, double *sm_clock_mhz);

@@ -40,7 +40,7 @@ SYMBOLS = ["socp_create", "socp_destroy", "socp_last_error", "socp_set_stream", 
            "socp_trace_width", "socp_trace_max_rows", "socp_trace_batch", "socp_point_batch", "socp_residual_batch", "socp_fdjac_batch", "socp_solve_batch",
            "socp_traj_var_batch", "socp_jacobian_batch", "socp_solve_hybrj_batch",
            "socp_continuation_param_batch", "socp_continuation_boundary_batch",
-           "socp_move_batch", "socp_solution_batch", "socp_measure_fp64_peak"]
+           "socp_move_batch", "socp_solution_batch", "socp_solution_trace_batch", "socp_measure_fp64_peak"]
 
 
 def lib():
@@ -88,6 +88,7 @@ def lib():
     L.socp_continuation_boundary_batch.argtypes = [vp, sp, cl, vp, vp, vp, vp, vp, vp, cd, ci, cd, cd, vp, vp, ci]
     L.socp_move_batch.argtypes = [vp, sp, cl, vp, vp, vp, ci, vp, vp, ci]
     L.socp_solution_batch.argtypes = [vp, sp, cl, vp, vp, vp, vp, vp, ci]
+    L.socp_solution_trace_batch.argtypes = [vp, sp, cl, vp, vp, vp, vp, vp, ci]
     L.socp_measure_fp64_peak.argtypes = [vp, P(cd), P(cd)]
     for name in SYMBOLS:
         f = getattr(L, name)

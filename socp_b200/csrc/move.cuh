@@ -1,4 +1,5 @@
-// socp_b200/csrc/move.cuh -- shooting::Move(tf) and shooting::GetSolution for a batch of solved problems.
+// socp_b200/csrc/move.cuh -- shooting::Move(tf), shooting::GetSolution and shooting::Trace for a batch of solved
+// problems.
 //
 // Restates shooting::Move(tf) (src/socp/shooting.cpp:383-437; cpp/src/socp/shooting.cpp:146-160) and
 // shooting::UpdateSolution (:1462-1508): the state of a solution at time t is the integration of the shooting
@@ -95,6 +96,32 @@ solution_nodes_kernel(MoveShape sh, long B, int N, const double *__restrict__ ti
             vX[b * (per + N) + r] = x[b * sh.P + r];
         }
     }
+}
+
+// shooting::Trace (src/socp/shooting.cpp:496-544): every segment of every solution re-integrated with the observer on.
+// rows[b][j] (R rows of W) = the rows of segment j of problem b, nrows[b * M + j] = their count: the trace_traj of
+// (tl[j], node j of x[b], tl[j + 1], switching times, S), so a segment is bit for bit the socp_trace_batch of the same
+// arguments.  The observer is the fixed-step RK4 one for every shape, SOCP_DOPRI5 included, as model::ModelInt's
+// trace branch (odeTools.cpp:103-123).  One thread per (problem, segment), 64-thread CTAs as trace_kernel.
+template <int MODEL>
+__global__ void __launch_bounds__(64)
+solution_trace_kernel(MoveShape sh, long B, int R, const double *__restrict__ mparams, const double *__restrict__ time,
+                      const double *__restrict__ x, double *__restrict__ rows, int *__restrict__ nrows) {
+    typedef Model<MODEL> M;
+    constexpr int N = M::N, W = N + M::NCTRL + 3;
+    const long w = (long)blockIdx.x * blockDim.x + threadIdx.x;
+    if (w >= B * sh.M) return;
+    const long b = w / sh.M;
+    const int j = (int)(w % sh.M);
+    const double *xb = x + b * sh.P;
+    const int nm = N * sh.M;
+    double t1, t2, sw[2] = {0.0227, 0.08};
+    timeline_pair(sh, time + b * (sh.M + 1), [&](int k) { return xb[nm + k]; }, j, t1, t2, sw);
+    typename M::Ctx c;
+    M::load(c, mparams + b * M::NP, sw);
+    double X[N];
+    for (int i = 0; i < N; ++i) X[i] = xb[N * j + i];
+    nrows[w] = trace_traj<MODEL>(c, X, t1, t2, sh.S, rows + w * R * W, W);
 }
 
 }  // namespace socp

@@ -394,6 +394,25 @@ class Engine:
                                                 a.out(vt), a.out(vX), mem))
         return vt, vX
 
+    def solution_trace_batch(self, shape, mparams, time, x):
+        """shooting::Trace for B solutions (socp_solution_trace_batch): returns (rows [B][M][R][W], nrows [B][M]),
+        rows[b, j, :nrows[b, j]] = the observer rows {t, X, control, H, extra} of segment j of problem b, RK4 for
+        every shape.  Numpy arrays or torch CUDA tensors, like solution_batch."""
+        mem, B, mparams = self._problem_args(shape, mparams, time, None, x)
+        M = shape.num_multi
+        W = self._L.socp_trace_width(shape.model_id)
+        R = self._L.socp_trace_max_rows(shape.model_id, int(shape.step_nbr))
+        if mem == HOST:
+            rows, nrows = np.empty((B, M, R, W)), np.empty((B, M), dtype=np.int32)
+        else:
+            import torch
+            rows = torch.empty((B, M, R, W), dtype=torch.float64, device=x.device)
+            nrows = torch.empty((B, M), dtype=torch.int32, device=x.device)
+        a = self._arg(mem)
+        self._check(self._L.socp_solution_trace_batch(self._h, ctypes.byref(shape), B, a.inp(mparams), a.inp(time),
+                                                      a.inp(x), a.out(rows), a.out(nrows, np.int32), mem))
+        return rows, nrows
+
     # -- analytic-Jacobian path (modelOrder == 1; the double integrator, as in the reference) -----
     def traj_var_batch(self, model_id, mparams, t0, X0, tf, step_nbr=0):
         """model::ComputeTraj(isJac = 1) for B extended states [(2dim+1) 2dim] (host arrays)."""
