@@ -189,24 +189,29 @@ static bool use_coop(socp_ctx *ctx, long items, int lanes) {
     return items * lanes <= (long)ctx->sm_count * 128 * 4;
 }
 
+// Calls f(std::bool_constant<ADAPTIVE>, std::integral_constant<int, L>) for the instance of an integrating kernel
+// that runs `items` work items: the adaptive integrator when tol > 0, L = Coop<MODEL>::LANES lanes per item when
+// use_coop says so, one otherwise.
+template <int MODEL, typename F>
+static void with_variant(socp_ctx *ctx, long items, double tol, F &&f) {
+    constexpr int L = Coop<MODEL>::LANES;
+    auto lanes = [&](auto adaptive) {
+        if (use_coop(ctx, items, L)) f(adaptive, std::integral_constant<int, L>());
+        else f(adaptive, std::integral_constant<int, 1>());
+    };
+    if (tol > 0.) lanes(std::true_type());
+    else lanes(std::false_type());
+}
+
 template <int MODEL>
 static void launch_traj(socp_ctx *ctx, long B, int S, const TrajIn &in, double *Xf, double tol, int *nsteps) {
-    const int threads = SOCP_TRAJ_THREADS;
-    constexpr int L = Coop<MODEL>::LANES;
-    if (use_coop(ctx, B, L)) {
-        const long blocks = (B * L + threads - 1) / threads;
-        if (tol > 0.)
-            traj_kernel<MODEL, true, L><<<(unsigned)blocks, threads, 0, ctx->stream>>>(B, S, in.mp, in.sw, in.t0, in.tf, in.X0, Xf, ctx->d_counters, tol, nsteps);
-        else
-            traj_kernel<MODEL, false, L><<<(unsigned)blocks, threads, 0, ctx->stream>>>(B, S, in.mp, in.sw, in.t0, in.tf, in.X0, Xf, ctx->d_counters, 0., nullptr);
-        ctx->launches += 1;
-        return;
-    }
-    long blocks = (B + threads - 1) / threads;
-    if (tol > 0.)
-        traj_kernel<MODEL, true><<<(unsigned)blocks, threads, 0, ctx->stream>>>(B, S, in.mp, in.sw, in.t0, in.tf, in.X0, Xf, ctx->d_counters, tol, nsteps);
-    else
-        traj_kernel<MODEL, false><<<(unsigned)blocks, threads, 0, ctx->stream>>>(B, S, in.mp, in.sw, in.t0, in.tf, in.X0, Xf, ctx->d_counters, 0., nullptr);
+    with_variant<MODEL>(ctx, B, tol, [&](auto adaptive, auto lanes) {
+        constexpr bool A = decltype(adaptive)::value;
+        constexpr int L = decltype(lanes)::value;
+        const long blocks = (B * L + SOCP_TRAJ_THREADS - 1) / SOCP_TRAJ_THREADS;
+        traj_kernel<MODEL, A, L><<<(unsigned)blocks, SOCP_TRAJ_THREADS, 0, ctx->stream>>>(
+            B, S, in.mp, in.sw, in.t0, in.tf, in.X0, Xf, ctx->d_counters, A ? tol : 0., A ? nsteps : nullptr);
+    });
     ctx->launches += 1;
 }
 

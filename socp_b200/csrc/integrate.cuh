@@ -21,13 +21,18 @@ namespace socp {
 // too small to fill the GPU with one thread per trajectory (the tail of a batched solve, small batches).
 template <int MODEL> struct Coop {
     static constexpr int LANES = 1;
-    SOCP_DEV static void set(typename Model<MODEL>::Ctx &, int, unsigned) {}
+    SOCP_DEV static void set(typename Model<MODEL>::Ctx &, int) {}
     SOCP_DEV static bool owns(const typename Model<MODEL>::Ctx &, int) { return true; }
     SOCP_DEV static double group_max(const typename Model<MODEL>::Ctx &, double v) { return v; }
 };
 template <> struct Coop<VTOL_UAV> {
     static constexpr int LANES = 4;
-    SOCP_DEV static void set(Model<VTOL_UAV>::Ctx &c, int q, unsigned mask) { c.coop_lanes = LANES; c.cq = q; c.cmask = mask; }
+    // lane q of the group of LANES consecutive lanes of the warp that holds this thread
+    SOCP_DEV static void set(Model<VTOL_UAV>::Ctx &c, int q) {
+        c.coop_lanes = LANES;
+        c.cq = q;
+        c.cmask = ((1u << LANES) - 1u) << ((threadIdx.x & 31) & ~(LANES - 1));
+    }
     SOCP_DEV static bool owns(const Model<VTOL_UAV>::Ctx &c, int i) { return c.coop_lanes == 1 || (i & (LANES - 1)) == c.cq; }
     // max over the group with MINPACK-free NaN semantics: a NaN anywhere gives NaN (the step is rejected)
     SOCP_DEV static double group_max(const Model<VTOL_UAV>::Ctx &c, double v) {
@@ -64,16 +69,24 @@ SOCP_DEV void rk4_step(const typename Model<MODEL>::Ctx &c, double t, double *X,
     for (int i = 0; i < N; ++i) X[i] = X[i] + h6 * (F1[i] + (F[i] + 2.0 * F23[i]));
 }
 
+// What a fixed-step integration reports besides its end point: nothing (NoRows), or the observer rows of a trace
+// (TraceRows, below).  Called at the start point and after every step.
+struct NoRows {
+    template <class C> SOCP_DEV void operator()(const C &, double, const double *) {}
+};
+
 // odeTools::integrate: `while (t < tf - dt/2)` with `t += dt` and a last-step clamp, so that
 // tf <= t0 performs zero steps.  Returns the number of RK4 steps taken.
-template <int MODEL>
-SOCP_DEV int integrate_fixed(const typename Model<MODEL>::Ctx &c, double *X, double t0, double tf, double dt) {
+template <int MODEL, class OBS>
+SOCP_DEV int integrate_fixed(const typename Model<MODEL>::Ctx &c, double *X, double t0, double tf, double dt, OBS &obs) {
     double t = t0;
     int steps = 0;
+    obs(c, t, X);
     while (t < (tf - dt / 2)) {
         rk4_step<MODEL>(c, t, X, (t + dt > tf) ? tf - t : dt);     // one inlined copy of the step
         t += dt;
         ++steps;
+        obs(c, t, X);
     }
     return steps;
 }
@@ -174,56 +187,55 @@ SOCP_DEV int integrate_adaptive(const typename Model<MODEL>::Ctx &c, double *X, 
     return steps;
 }
 
-// model::ComputeTraj for one segment.  For the interceptor `c.chart` / `c.stage` are updated and
-// left as the reference leaves its hidden state (the final state is converted back to chart 1
-// but currentChart is not reset, interceptor.cpp:214-216).
-template <int MODEL>
-SOCP_DEV int compute_traj(typename Model<MODEL>::Ctx &c, double *X, double t0, double tf, int S) {
-    return integrate_fixed<MODEL>(c, X, t0, tf, (tf - t0) / S);
-}
-
-SOCP_DEV int interceptor_model_int(Model<INTERCEPTOR>::Ctx &c, double *X, double t0, double tf, int S) {
+template <class OBS>
+SOCP_DEV int interceptor_model_int(Model<INTERCEPTOR>::Ctx &c, double *X, double t0, double tf, int S, OBS &obs) {
     double t = t0;
     const double dt = (tf - t0) / S;
+    obs(c, t, X);
     for (int i = 0; i < S; ++i) {
         Model<INTERCEPTOR>::set_chart(c, X);
         rk4_step<INTERCEPTOR>(c, t, X, dt);
         t += dt;
+        obs(c, t, X);
     }
     return S;
 }
 
-template <>
-SOCP_DEV int compute_traj<INTERCEPTOR>(Model<INTERCEPTOR>::Ctx &c, double *X, double t0, double tf, int S) {
-    int steps = 0;
-    c.chart = 1;
-    const double t1 = c.mprop / c.q;
-    if (t0 < t1) {
-        c.stage = 1;
-        if (tf > t1) {
-            steps += interceptor_model_int(c, X, t0, t1, S);
-            c.stage = 0;
-            steps += interceptor_model_int(c, X, t1, tf, S);
+// model::ComputeTraj for one segment.  For the interceptor `c.chart` / `c.stage` are updated and
+// left as the reference leaves its hidden state (the final state is converted back to chart 1
+// but currentChart is not reset, interceptor.cpp:214-216).
+template <int MODEL, class OBS = NoRows>
+SOCP_DEV int compute_traj(typename Model<MODEL>::Ctx &c, double *X, double t0, double tf, int S, OBS &&obs = OBS()) {
+    if constexpr (MODEL == INTERCEPTOR) {
+        int steps = 0;
+        c.chart = 1;
+        const double t1 = c.mprop / c.q;
+        if (t0 < t1) {
+            c.stage = 1;
+            if (tf > t1) {
+                steps += interceptor_model_int(c, X, t0, t1, S, obs);
+                c.stage = 0;
+                steps += interceptor_model_int(c, X, t1, tf, S, obs);
+            } else {
+                steps += interceptor_model_int(c, X, t0, tf, S, obs);
+            }
         } else {
-            steps += interceptor_model_int(c, X, t0, tf, S);
+            c.stage = 0;
+            steps += interceptor_model_int(c, X, t0, tf, S, obs);
         }
+        if (c.chart == 2) Model<INTERCEPTOR>::convert(2, X);
+        return steps;
     } else {
-        c.stage = 0;
-        steps += interceptor_model_int(c, X, t0, tf, S);
+        return integrate_fixed<MODEL>(c, X, t0, tf, (tf - t0) / S, obs);
     }
-    if (c.chart == 2) Model<INTERCEPTOR>::convert(2, X);
-    return steps;
 }
 
 // model::ComputeTraj with the adaptive integrator (the reference's Boost build).  The interceptor keeps
 // its own fixed-step loop there too (interceptor.cpp:104-130 calls RK4 directly).
 template <int MODEL>
 SOCP_DEV int compute_traj_adaptive(typename Model<MODEL>::Ctx &c, double *X, double t0, double tf, int S, double tol, int &rejected) {
-    return integrate_adaptive<MODEL>(c, X, t0, tf, (tf - t0) / S, tol, rejected);
-}
-template <>
-SOCP_DEV int compute_traj_adaptive<INTERCEPTOR>(Model<INTERCEPTOR>::Ctx &c, double *X, double t0, double tf, int S, double, int &) {
-    return compute_traj<INTERCEPTOR>(c, X, t0, tf, S);
+    if constexpr (MODEL == INTERCEPTOR) return compute_traj<MODEL>(c, X, t0, tf, S);
+    else return integrate_adaptive<MODEL>(c, X, t0, tf, (tf - t0) / S, tol, rejected);
 }
 
 template <int MODEL> SOCP_DEV void get_chart_stage(const typename Model<MODEL>::Ctx &, int &chart, int &stage) { chart = 1; stage = 0; }
@@ -265,7 +277,7 @@ traj_kernel(long B, int S, const double *__restrict__ mparams, const double *__r
     if (b < B) {
         typename M::Ctx c;
         M::load(c, mparams + b * M::NP, sw ? sw + 2 * b : nullptr);
-        if (L > 1) Coop<MODEL>::set(c, q, ((1u << L) - 1u) << ((threadIdx.x & 31) & ~(L - 1)));
+        if (L > 1) Coop<MODEL>::set(c, q);
         double X[N];
 #pragma unroll
         for (int i = 0; i < N; ++i) X[i] = X0[b * N + i];
@@ -305,55 +317,20 @@ __device__ __noinline__ void trace_row(const typename Model<MODEL>::Ctx &c, doub
     row[2 + N + M::NCTRL] = trace_extra<MODEL>(c, X);
 }
 
+template <int MODEL> struct TraceRows {
+    double *rows;
+    int W, n;
+    SOCP_DEV void operator()(const typename Model<MODEL>::Ctx &c, double t, const double *X) {
+        trace_row<MODEL>(c, t, X, rows + (size_t)(n++) * W);
+    }
+};
+
+// compute_traj with the observer on: returns the rows written (S + 1 per integration)
 template <int MODEL>
 SOCP_DEV int trace_traj(typename Model<MODEL>::Ctx &c, double *X, double t0, double tf, int S, double *rows, int W) {
-    const double dt = (tf - t0) / S;
-    double t = t0;
-    int nr = 0;
-    trace_row<MODEL>(c, t, X, rows + (size_t)(nr++) * W);
-    while (t < (tf - dt / 2)) {
-        if (t + dt > tf) rk4_step<MODEL>(c, t, X, tf - t);
-        else rk4_step<MODEL>(c, t, X, dt);
-        t += dt;
-        trace_row<MODEL>(c, t, X, rows + (size_t)(nr++) * W);
-    }
-    return nr;
-}
-
-SOCP_DEV int interceptor_trace_int(Model<INTERCEPTOR>::Ctx &c, double *X, double t0, double tf, int S, double *rows, int W) {
-    double t = t0;
-    const double dt = (tf - t0) / S;
-    int nr = 0;
-    trace_row<INTERCEPTOR>(c, t, X, rows + (size_t)(nr++) * W);
-    for (int i = 0; i < S; ++i) {
-        Model<INTERCEPTOR>::set_chart(c, X);
-        rk4_step<INTERCEPTOR>(c, t, X, dt);
-        t += dt;
-        trace_row<INTERCEPTOR>(c, t, X, rows + (size_t)(nr++) * W);
-    }
-    return nr;
-}
-
-template <>
-SOCP_DEV int trace_traj<INTERCEPTOR>(Model<INTERCEPTOR>::Ctx &c, double *X, double t0, double tf, int S, double *rows, int W) {
-    int nr = 0;
-    c.chart = 1;
-    const double t1 = c.mprop / c.q;
-    if (t0 < t1) {
-        c.stage = 1;
-        if (tf > t1) {
-            nr += interceptor_trace_int(c, X, t0, t1, S, rows, W);
-            c.stage = 0;
-            nr += interceptor_trace_int(c, X, t1, tf, S, rows + (size_t)nr * W, W);
-        } else {
-            nr += interceptor_trace_int(c, X, t0, tf, S, rows, W);
-        }
-    } else {
-        c.stage = 0;
-        nr += interceptor_trace_int(c, X, t0, tf, S, rows, W);
-    }
-    if (c.chart == 2) Model<INTERCEPTOR>::convert(2, X);
-    return nr;
+    TraceRows<MODEL> obs{rows, W, 0};
+    compute_traj<MODEL>(c, X, t0, tf, S, obs);
+    return obs.n;
 }
 
 // rows: [B][max_rows][W]; nrows[b] = rows written (S+1 per integration, two integrations for a

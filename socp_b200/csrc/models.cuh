@@ -33,12 +33,14 @@ template <> struct Model<GODDARD> {
     static constexpr int DIM = 7, N = 14, NP = 8, NCTRL = 3, DEFAULT_STEPS = 10;
     static constexpr int MINB = 1;      // CTAs/SM asked of the trajectory kernels: 240 registers, no spills (a cap of 168 costs 30%)
     struct Ctx { double C, b, KD, kr, umax, mu1, mu2, sing, sw0, sw1, half_inv_mu2; };
+    // the switching times before the first SwitchingTimesUpdate (goddard.cpp:27-29)
+    static constexpr double SW0_GUESS = 0.0227, SW1_GUESS = 0.08;
     SOCP_DEV static void load(Ctx &c, const double *m, const double *sw) {
         c.C = m[0]; c.b = m[1]; c.KD = m[2]; c.kr = m[3]; c.umax = m[4]; c.mu1 = m[5]; c.mu2 = m[6];
         c.sing = m[7];
         c.half_inv_mu2 = 0.5 / c.mu2;     // hoisted out of the RHS: alpha_u = -Switch / 2 / mu2
-        c.sw0 = sw ? sw[0] : 0.0227;      // goddard.cpp:27-29
-        c.sw1 = sw ? sw[1] : 0.08;
+        c.sw0 = sw ? sw[0] : SW0_GUESS;
+        c.sw1 = sw ? sw[1] : SW1_GUESS;
     }
 
     // goddard.cpp:188-253 (true singular control), expression order of the reference.  Out of line:

@@ -42,7 +42,7 @@ move_kernel(MoveShape sh, long B, int Q, const double *__restrict__ mparams, con
         const int nm = N * sh.M;
         auto xfree = [&](int k) { return xb[nm + k]; };
         // ComputeTimeLine first, as the reference's Move does: t0, t_end and the switching times
-        double t1, t2, t_end, sw[2] = {0.0227, 0.08}, sw_unused[2];
+        double t1, t2, t_end, sw[2] = {Model<GODDARD>::SW0_GUESS, Model<GODDARD>::SW1_GUESS}, sw_unused[2];
         timeline_pair(sh, time_b, xfree, sh.M - 1, t1, t_end, sw);
         timeline_pair(sh, time_b, xfree, 0, t1, t2, sw_unused);
         // a query outside [t0, t_end] (NaN included) is answered at t_end
@@ -56,7 +56,7 @@ move_kernel(MoveShape sh, long B, int Q, const double *__restrict__ mparams, con
         }
         typename M::Ctx c;
         M::load(c, mparams + b * M::NP, sw);
-        if (L > 1) Coop<MODEL>::set(c, lane, ((1u << L) - 1u) << ((threadIdx.x & 31) & ~(L - 1)));
+        if (L > 1) Coop<MODEL>::set(c, lane);
         double X[N];
 #pragma unroll
         for (int i = 0; i < N; ++i) X[i] = xb[N * seg + i];
@@ -115,10 +115,9 @@ solution_trace_kernel(MoveShape sh, long B, int R, const double *__restrict__ mp
     const int j = (int)(w % sh.M);
     const double *xb = x + b * sh.P;
     const int nm = N * sh.M;
-    double t1, t2, sw[2] = {0.0227, 0.08};
-    timeline_pair(sh, time + b * (sh.M + 1), [&](int k) { return xb[nm + k]; }, j, t1, t2, sw);
+    double t1, t2;
     typename M::Ctx c;
-    M::load(c, mparams + b * M::NP, sw);
+    segment_setup<MODEL>(sh, time + b * (sh.M + 1), [&](int k) { return xb[nm + k]; }, j, mparams + b * M::NP, t1, t2, c);
     double X[N];
     for (int i = 0; i < N; ++i) X[i] = xb[N * j + i];
     nrows[w] = trace_traj<MODEL>(c, X, t1, t2, sh.S, rows + w * R * W, W);

@@ -168,26 +168,8 @@ template <int G> SOCP_DEV double enorm_g(int n, const double *x, double *) {
 // Node times from the fixed times and the FREE-time unknowns, linear interpolation for CONTINUOUS
 // nodes.  xfree(k) returns the k-th free-time unknown (already perturbed if needed).
 // sw[2] receives the first two FREE interior times (SwitchingTimesUpdate, goddard.cpp:373).
-template <class XF>
-SOCP_DEV void timeline_all(const SolverDev &D, const double *time_b, XF xfree, double *tl, double *sw) {
-    int k = 0, cur = 0, nsw = 0;
-    for (int j = 0; j <= D.M; ++j) {
-        const int m = D.mode_t[j];
-        if (m == SOCP_FIXED || m == SOCP_FREE) {
-            double tj;
-            if (m == SOCP_FIXED) tj = time_b[j];
-            else {
-                tj = xfree(k++);
-                if (j < D.M && nsw < 2) sw[nsw++] = tj;
-            }
-            tl[j] = tj;
-            for (int q = cur + 1; q < j; ++q) tl[q] = tl[cur] + (q - cur) * (tl[j] - tl[cur]) / (j - cur);
-            cur = j;
-        }
-    }
-}
-// the two node times of segment s without materialising the whole line.  SH is any shape with M and mode_t[M + 1]:
-// SolverDev for the solver kernels, MoveShape for the move kernel (move.cuh).
+// t1, t2 = the two node times of segment s, without materialising the whole line.  SH is any shape with M and
+// mode_t[M + 1]: SolverDev for the solver kernels, MoveShape for the move kernels (move.cuh).
 template <class SH, class XF>
 SOCP_DEV void timeline_pair(const SH &D, const double *time_b, XF xfree, int s, double &t1, double &t2, double *sw) {
     int k = 0, cur = 0, nsw = 0;
@@ -210,6 +192,17 @@ SOCP_DEV void timeline_pair(const SH &D, const double *time_b, XF xfree, int s, 
             tcur = tj;
         }
     }
+}
+
+// Segment s of a problem as its integration starts: the node times t1, t2 and the model context loaded from the
+// parameter block mp with the switching times of the time line (Goddard's guesses while it has fewer than two FREE
+// interior times; the other models ignore them).
+template <int MODEL, class SH, class XF>
+SOCP_DEV void segment_setup(const SH &D, const double *time_b, XF xfree, int s, const double *mp, double &t1, double &t2,
+                            typename Model<MODEL>::Ctx &c) {
+    double sw[2] = {Model<GODDARD>::SW0_GUESS, Model<GODDARD>::SW1_GUESS};
+    timeline_pair(D, time_b, xfree, s, t1, t2, sw);
+    Model<MODEL>::load(c, mp, sw);
 }
 
 // MINPACK fdjac1 step for unknown value v
@@ -259,12 +252,11 @@ integrate_worklist(SolverDev D, int cur) {
         const double *xe = D.xe + b * D.P;
         const double h = (col >= 0) ? fd_step(xe[col], D.epsfcn) : 0.0;
         const int nm = N * D.M;
-        double t1, t2, sw[2] = {0.0227, 0.08};
-        timeline_pair(D, D.time + b * (D.M + 1),
-                      [&](int k) { int idx = nm + k; return xe[idx] + ((idx == col) ? h : 0.0); }, s, t1, t2, sw);
+        double t1, t2;
         typename M::Ctx c;
-        M::load(c, D.mparams + b * M::NP, sw);
-        if (L > 1) Coop<MODEL>::set(c, cq, ((1u << L) - 1u) << ((threadIdx.x & 31) & ~(L - 1)));
+        segment_setup<MODEL>(D, D.time + b * (D.M + 1), [&](int k) { int idx = nm + k; return xe[idx] + ((idx == col) ? h : 0.0); },
+                             s, D.mparams + b * M::NP, t1, t2, c);
+        if (L > 1) Coop<MODEL>::set(c, cq);
         double X[N];
 #pragma unroll
         for (int i = 0; i < N; ++i) X[i] = xe[N * s + i];
@@ -327,14 +319,12 @@ __device__ __noinline__ void assemble(const SolverDev &D, long b, int col, doubl
     };
     // node times on demand (timeline_pair per evaluated segment: no per-thread array of M + 1 times in local memory);
     // the first call also yields the switching times the model context needs
-    double sw[2] = {0.0227, 0.08};
     const int nm = N * D.M;
     const double *time_b = D.time + b * (D.M + 1);
     auto xfree = [&](int k) { return xv(nm + k); };
     double t_lo, t_hi;
-    timeline_pair(D, time_b, xfree, seg_lo, t_lo, t_hi, sw);
     typename M::Ctx c;
-    M::load(c, mp, sw);
+    segment_setup<MODEL>(D, time_b, xfree, seg_lo, mp, t_lo, t_hi, c);
     int nbr = nm;
     double X1[N], Xtf[N], Xp[N];
     for (int i = 0; i < D.M; ++i) {
@@ -583,10 +573,9 @@ integrate_var_worklist(SolverDev D, int cur) {
         if (i >= N) continue;
         const double *xe = D.xe + b * D.P;
         const int nm = N * D.M;
-        double t1, t2, sw[2] = {0.0227, 0.08};
-        timeline_pair(D, D.time + b * (D.M + 1), [&](int k) { return xe[nm + k]; }, s, t1, t2, sw);
+        double t1, t2;
         typename M::Ctx c;
-        M::load(c, D.mparams + b * M::NP, sw);
+        segment_setup<MODEL>(D, D.time + b * (D.M + 1), [&](int k) { return xe[nm + k]; }, s, D.mparams + b * M::NP, t1, t2, c);
         double X[N], phi[N];
 #pragma unroll
         for (int k = 0; k < N; ++k) { X[k] = xe[N * s + k]; phi[k] = (k == i) ? 1. : 0.; }
@@ -617,15 +606,15 @@ assemble_jac_kernel(SolverDev D, int cur) {
     for (long w = (long)blockIdx.x * blockDim.x + threadIdx.x; w < njac; w += (long)gridDim.x * blockDim.x) {
         const long b = jac_list[w];
         const double *xe = D.xe + b * P;
-        const double *mp = D.mparams + b * M::NP;
         double *J = D.fjac + (size_t)b * D.QS;
         auto put = [&](int row, int col, double v) { J[row + (size_t)col * P] = v; };     // dF_row / dx_col
         for (int e = 0; e < P * P; ++e) J[e] = 0.;
-        double tl[SOCP_MAX_NODES + 1], sw[2] = {0.0227, 0.08};
         const int nm = N * D.M;
-        timeline_all(D, D.time + b * (D.M + 1), [&](int k) { return xe[nm + k]; }, tl, sw);
+        const double *time_b = D.time + b * (D.M + 1);
+        auto xfree = [&](int k) { return xe[nm + k]; };
         typename M::Ctx c;
-        M::load(c, mp, sw);
+        double t1, t2;      // the node times of segment i in the loop below
+        segment_setup<MODEL>(D, time_b, xfree, 0, D.mparams + b * M::NP, t1, t2, c);
         int nbr = nm;
         // rows of a boundary function: FIXED component j -> sensitivity row j, FREE -> row j + n; with a
         // free time one more column (the flow) and one more row (dH) (model.hpp:104-120, :149-183)
@@ -650,13 +639,14 @@ assemble_jac_kernel(SolverDev D, int cur) {
             }
         };
         for (int i = 0; i < D.M; ++i) {
-            const double t2 = tl[i + 1];
+            double sw_unused[2];
+            timeline_pair(D, time_b, xfree, i, t1, t2, sw_unused);
             const double *seg = D.jends + ((size_t)b * D.M + i) * NV;     // X(t2) and Phi = dX(t2)/dX(t1)
             const double *Xtf = seg, *Phi = seg + N;                      // Phi[N k + q] = dX_k / dX0_q
             const int index = N * (i + 1);
             if (i == 0) {
                 const bool withH = D.mode_t[0] != SOCP_FIXED;
-                boundary(xe, nullptr, tl[0], D.mode_X[0], true, 0, 0, withH);
+                boundary(xe, nullptr, t1, D.mode_X[0], true, 0, 0, withH);
                 if (withH) nbr += 1;
             }
             if (i < D.M - 1) {
