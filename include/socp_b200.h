@@ -113,6 +113,10 @@ int socp_model_nparams(int model_id);
 int socp_model_default_steps(int model_id);
 int socp_model_default_params(int model_id, double *out);     /* constructor defaults */
 int socp_num_param(const socp_shape *shape);                   /* shooting.cpp:179,196 */
+/* the structural band of the shape's shooting Jacobian: rows [lo[j], end[j]) of column j (P entries each) hold every
+ * entry that the forward-difference Jacobian and its Householder QR can make non-zero.  Returns 1 when the solver's
+ * Jacobian phase works on the band instead of the dense matrix, 0 when not, < 0 for a bad shape. */
+int socp_jac_band(const socp_shape *shape, int *lo, int *end);
 
 /* obstacle table of the vtolUAV penalty map (src/maps/obstacle/obstacle.cpp:24-36): type 0 ellipsoid,
  * 1 box; pos/rad are [n][3], host pointers.  The table lives in constant memory of the DEVICE: it is

@@ -36,7 +36,7 @@ _LIB = None
 SYMBOLS = ["socp_create", "socp_destroy", "socp_last_error", "socp_set_stream", "socp_sync",
            "socp_get_stats", "socp_reset_stats", "socp_set_profiling", "socp_timer_start", "socp_timer_stop",
            "socp_model_dim", "socp_model_nparams", "socp_model_default_steps",
-           "socp_model_default_params", "socp_num_param", "socp_set_obstacles", "socp_traj_batch", "socp_traj_adaptive_batch",
+           "socp_model_default_params", "socp_num_param", "socp_jac_band", "socp_set_obstacles", "socp_traj_batch", "socp_traj_adaptive_batch",
            "socp_trace_width", "socp_trace_max_rows", "socp_trace_batch", "socp_point_batch", "socp_residual_batch", "socp_fdjac_batch", "socp_solve_batch",
            "socp_traj_var_batch", "socp_jacobian_batch", "socp_solve_hybrj_batch",
            "socp_continuation_param_batch", "socp_continuation_boundary_batch",
@@ -71,6 +71,7 @@ def lib():
     L.socp_model_default_steps.argtypes = [ci]
     L.socp_model_default_params.argtypes = [ci, vp]
     L.socp_num_param.argtypes = [sp]
+    L.socp_jac_band.argtypes = [sp, vp, vp]
     L.socp_set_obstacles.argtypes = [vp, ci, vp, vp, vp]
     L.socp_traj_batch.argtypes = [vp, ci, ci, cl, vp, vp, vp, vp, vp, vp, ci]
     L.socp_traj_adaptive_batch.argtypes = [vp, ci, ci, cl, vp, vp, vp, vp, vp, cd, vp, vp, ci]

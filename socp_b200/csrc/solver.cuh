@@ -47,6 +47,9 @@ struct SolverDev {
     int mode_X[SOCP_MAX_NODES][SOCP_MAX_DIM];
     const int *jac_col, *jac_seg;          // [nJ] work item -> (column, segment)
     const int *col_item0, *col_nseg;       // [P] first item of a column; 1 or M segments
+    const int *band_lo, *band_off;         // [P], [P + 1] structural band of the Jacobian (jac_band): column k keeps the
+                                           // rows band_lo[k] .. band_lo[k] + band_off[k + 1] - band_off[k] - 1
+    int band_doubles;                      // > 0: the Jacobian phase runs hybrd_jac_band_kernel on a band of this size
     // problem data
     long B;
     const double *mparams, *time, *Xb;
@@ -119,17 +122,21 @@ SOCP_DEV double warp_max_d(double v) {
 // intermediate range are summed as plain squares; small (<= rdwarf) and large (>= rgiant/n) ones are
 // scaled by their maximum as MINPACK does, but with the maximum found first (a reduction) instead
 // of by running rescaling, so nothing is sequential.  Every lane returns the same value.
-SOCP_DEV double enorm_warp(int n, const double *x) {
+// enorm_rows: the same norm of an n-vector whose components outside [lo, end) are zeros and not stored
+// (x[i - lo] is component i).  Component i stays on lane i % 32, so the bits are those of the full vector: a
+// zero adds nothing to any of the sums.
+SOCP_DEV double enorm_rows(int n, const double *x, int lo, int end) {
     const double rdwarf = 3.834e-20, rgiant = 1.304e19;
     // MINPACK's agiant = rgiant / n; the range test is written xabs * n < rgiant so that no call pays a
     // divide (the two differ only for a component within an ulp of the threshold, where either
     // accumulation is safe)
     const double dn = (double)n;
     const int lane = threadIdx.x & 31;
+    const int first = lo + ((lane - lo) & 31);
     double s2 = 0., small_max = 0., big_max = 0.;
     bool isnan_ = false;
-    for (int i = lane; i < n; i += 32) {
-        const double xabs = fabs(x[i]);
+    for (int i = first; i < end; i += 32) {
+        const double xabs = fabs(x[i - lo]);
         if (xabs > rdwarf && xabs * dn < rgiant) s2 = fma(xabs, xabs, s2);
         else if (xabs <= rdwarf) small_max = fmax(small_max, xabs);
         else if (xabs == xabs) big_max = fmax(big_max, xabs);
@@ -141,8 +148,8 @@ SOCP_DEV double enorm_warp(int n, const double *x) {
     if (!special) return sqrt(s2);
     const double x1max = warp_max_d(big_max), x3max = warp_max_d(small_max);
     double s1 = 0., s3 = 0.;
-    for (int i = lane; i < n; i += 32) {
-        const double xabs = fabs(x[i]);
+    for (int i = first; i < end; i += 32) {
+        const double xabs = fabs(x[i - lo]);
         if (xabs > rdwarf && xabs * dn < rgiant) continue;
         if (xabs <= rdwarf) { if (xabs != 0.) { const double q = xabs / x3max; s3 = fma(q, q, s3); } }
         else { const double q = xabs / x1max; s1 = fma(q, q, s1); }
@@ -156,6 +163,7 @@ SOCP_DEV double enorm_warp(int n, const double *x) {
     }
     return x3max * sqrt(s3);
 }
+SOCP_DEV double enorm_warp(int n, const double *x) { return enorm_rows(n, x, 0, n); }
 
 // Euclidean norm over a thread group: every warp of the group evaluates enorm_warp on the whole
 // vector (n is a few hundred at most), so no block-level reduction or barrier is needed and every
@@ -772,6 +780,23 @@ SOCP_DEV void axpy_sub4(double *y, const double *x, double t, int m) {
     for (; i < m; ++i) y[i] = __fma_rn(-t, x[i], y[i]);
 }
 
+// Column layouts of the matrix the Jacobian phase factors.  at(k, i) is the element in row i of column k; the rows of
+// column k outside [lo(k), end(k)) are exact zeros and are not stored.
+struct DenseCols {                       // column-major, leading dimension lda
+    double *a;
+    int lda, n;
+    SOCP_DEV double *at(int k, int i) const { return a + i + (size_t)k * lda; }
+    SOCP_DEV int lo(int) const { return 0; }
+    SOCP_DEV int end(int) const { return n; }
+};
+struct BandCols {                        // the structural band of SolverDev::band_lo / band_off, columns back to back
+    double *a;
+    const int *lo_, *off_;
+    SOCP_DEV double *at(int k, int i) const { return a + off_[k] + (i - lo_[k]); }
+    SOCP_DEV int lo(int k) const { return lo_[k]; }
+    SOCP_DEV int end(int k) const { return lo_[k] + (off_[k + 1] - off_[k]); }
+};
+
 // qrfac (no pivoting) fused with "qtf = Q^T fvec" (the Householder reflections are applied to
 // qtf as one more column); rdiag/acnorm as in MINPACK.  One thread per column.
 // Both routines skip work on EXACT zeros: hi[k] is the last row of column k that is not an exact zero
@@ -779,45 +804,49 @@ SOCP_DEV void axpy_sub4(double *y, const double *x, double t, int m) {
 // lower band), so reflector j only spans rows j..hi[j] and a column whose dot product with it is an
 // exact zero is left alone.  The skipped operations would add or subtract exact zeros: the factors are
 // the ones the dense MINPACK loops produce (up to the sign of a zero).
-template <int G>
-__device__ void qrfac_g(int n, double *a, int lda, double *rdiag, double *acnorm, double *qtf, double *red, int rot, int *hi) {
+// With a BandCols layout, a column whose stored rows do not hold all of rows j..hi[j] is one the reflector cannot
+// reach (the band holds every row that fill-in can reach, jac_band): its dot product would be an exact zero.
+template <int G, class C>
+__device__ void qrfac_g(int n, C a, double *rdiag, double *acnorm, double *qtf, double *red, int rot, int *hi) {
     // `rot` rotates the warp that owns the first columns: the active columns always start at thread 0, so
     // without it the co-resident CTAs of an SM would all load the same scheduler (see seq_warp)
     const int tid = (threadIdx.x + 32 * rot) % G;
     gsync<G>();
     for (int j = tid >> 5; j < n; j += G / 32) {       // column norms, one warp per column
-        const double v = enorm_warp(n, a + (size_t)j * lda);
+        const double v = enorm_rows(n, a.at(j, a.lo(j)), a.lo(j), a.end(j));
         if ((tid & 31) == 0) acnorm[j] = v;
     }
     for (int k = tid; k <= n; k += G) {                // last non-zero row of every column (qtf: dense)
         int last = (k < n) ? 0 : n - 1;
         if (k < n) {
-            const double *ck = a + (size_t)k * lda;
-            for (int i = n - 1; i > 0; --i) if (ck[i] != 0.) { last = i; break; }
+            const int lo = a.lo(k);
+            const double *ck = a.at(k, lo);
+            for (int i = a.end(k) - 1; i > 0 && i >= lo; --i) if (ck[i - lo] != 0.) { last = i; break; }
         }
         hi[k] = last;
     }
     gsync<G>();
     for (int j = 0; j < n; ++j) {
-        double *cj = a + (size_t)j * lda;
+        double *cj = a.at(j, j);                       // rows j .. hj of the reflector
         const int hj = max(hi[j], j), len = hj - j + 1;
-        double ajnorm = enorm_g<G>(len, cj + j, red);
+        double ajnorm = enorm_g<G>(len, cj, red);
         if (ajnorm != 0.) {
-            if (cj[j] < 0.) ajnorm = -ajnorm;
+            if (cj[0] < 0.) ajnorm = -ajnorm;
             gsync<G>();
-            for (int i = j + tid; i <= hj; i += G) {
+            for (int i = tid; i < len; i += G) {
                 double v = cj[i] / ajnorm;
-                if (i == j) v += 1.;
+                if (i == 0) v += 1.;
                 cj[i] = v;
             }
             gsync<G>();
-            const double ajj = cj[j];
+            const double ajj = cj[0];
             for (int k = j + 1 + tid; k <= n; k += G) {  // remaining columns, and qtf as column n
-                double *ck = (k < n) ? a + (size_t)k * lda : qtf;
-                const double sum = dot4(cj + j, ck + j, len);
+                if (k < n && (j < a.lo(k) || hj >= a.end(k))) continue;
+                double *ck = (k < n) ? a.at(k, j) : qtf + j;
+                const double sum = dot4(cj, ck, len);
                 if (sum != 0.) {
                     const double temp = sum / ajj;
-                    axpy_sub4(ck + j, cj + j, temp, len);
+                    axpy_sub4(ck, cj, temp, len);
                     if (hi[k] < hj) hi[k] = hj;
                 }
             }
@@ -874,8 +903,8 @@ SOCP_DEV bool window_ok(int n, int NB, const int *hi, int *flag) {
         (sum) = (s0_ + s1_) + (s2_ + s3_);                                                        \
     } while (0)
 
-template <int G, int NB>
-__device__ void qform_p(int n, const double *a, int lda, const int *hi, double *gq) {
+template <int G, int NB, class C>
+__device__ void qform_p(int n, C a, const int *hi, double *gq) {
     constexpr int W = 2 * NB;
     const int j = threadIdx.x % G;                 // this thread's column of Q
     if (j >= n) return;
@@ -894,7 +923,7 @@ __device__ void qform_p(int n, const double *a, int lda, const int *hi, double *
         for (int kk = NB - 1; kk >= 0; --kk) {
             const int k = c0 + kk;
             if (k > j || k >= n) continue;
-            const double *v = a + (size_t)k * lda + c0;        // v[t] = reflector k at row c0 + t (t >= kk)
+            const double *v = a.at(k, k) - kk;                 // v[t] = reflector k at row c0 + t (t >= kk)
             const double wk = v[kk];
             if (wk == 0.) continue;                            // the identity
             const int len = max(hi[k], k) - k + 1;             // rows k .. hk; exact zeros below
@@ -923,13 +952,15 @@ __device__ void qform_p(int n, const double *a, int lda, const int *hi, double *
     }
 }
 
-// copy R into packed storage (upper triangle by rows), diagonal from rdiag
-template <int G>
-__device__ void pack_r_g(int n, const double *a, int lda, const double *rdiag, double *r) {
+// copy R into packed storage (upper triangle by rows), diagonal from rdiag; the rows above a column's stored
+// ones are zeros
+template <int G, class C>
+__device__ void pack_r_g(int n, C a, const double *rdiag, double *r) {
     const int tid = threadIdx.x % G;
     for (int j = tid; j < n; j += G) {
         int l = j;
-        for (int i = 0; i < j; ++i) { r[l] = a[i + (size_t)j * lda]; l += n - 1 - i; }
+        const int lo = a.lo(j);
+        for (int i = 0; i < j; ++i) { r[l] = (i < lo) ? 0. : *a.at(j, i); l += n - 1 - i; }
         r[l] = rdiag[j];
     }
     gsync<G>();
@@ -1875,9 +1906,11 @@ hybrd_chain_kernel(SolverDev D, int cur, int per_group_doubles) {
 }
 
 // ---- kernel 2c: problems whose forward-difference Jacobian arrived ------------------------------
-template <int G, bool STAGE_R, bool STAGE_Q>
-__global__ void __launch_bounds__(128, 3)      // three CTAs per SM is what shared memory allows at P = 85: 168 registers
-hybrd_jac_kernel(SolverDev D, int cur, int per_group_doubles) {
+// BAND: the matrix is staged as its structural band (SolverDev::band_lo / band_off) after the 13 P work vectors, then
+// the two tables; R stays in global memory and qform_p writes Q there.
+template <int G, bool STAGE_R, bool STAGE_Q, bool BAND>
+SOCP_DEV void jac_loop(const SolverDev &D, int cur, int per_group_doubles) {
+    static_assert(!BAND || (STAGE_Q && !STAGE_R), "the banded Jacobian phase stages the matrix and leaves R in global memory");
     const int GROUPS = (G == 32) ? (int)(blockDim.x >> 5) : 1;
     const int grp = (G == 32) ? (threadIdx.x >> 5) : 0;
     const int tid = threadIdx.x % G;
@@ -1891,7 +1924,15 @@ hybrd_jac_kernel(SolverDev D, int cur, int per_group_doubles) {
     int *next_cnt = D.counts + (1 - cur) * 2;
     const int ldq_s = n | 1;                               // odd leading dimension in shared memory
     // 128-thread CTA, Q staged: Q travels by bulk copy when its shared layout equals the global one (odd P)
-    const bool bulk = (G == 128) && STAGE_Q && ldq_s == n;
+    const bool bulk = (G == 128) && STAGE_Q && !BAND && ldq_s == n;
+    int *band_lo = (int *)(vec + 13 * n + D.band_doubles), *band_off = band_lo + n;
+    if (BAND) {
+        for (int k = tid; k <= n; k += G) {
+            if (k < n) band_lo[k] = D.band_lo[k];
+            band_off[k] = D.band_off[k];
+        }
+    }
+    const BandCols band{vec + 13 * n, band_lo, band_off};
     __shared__ unsigned long long jac_bar;
     unsigned jac_parity = 0;
     if (bulk) {
@@ -1926,7 +1967,12 @@ hybrd_jac_kernel(SolverDev D, int cur, int per_group_doubles) {
                 mbar_expect_tx(&jac_bar, (unsigned)D.QS * 8u);
                 bulk_g2s(W.q, gq, (unsigned)D.QS * 8u, &jac_bar);
             }
-        } else if (STAGE_Q)
+        } else if (BAND)
+            for (int c = tid >> 5; c < n; c += G / 32) {
+                const int lo = band_lo[c], len = band_off[c + 1] - band_off[c];
+                for (int i = tid & 31; i < len; i += 32) __pipeline_memcpy_async(band.a + band_off[c] + i, gq + lo + i + (size_t)c * n, sizeof(double));
+            }
+        else if (STAGE_Q)
             for (int c = tid >> 5; c < n; c += G / 32)
                 for (int i = tid & 31; i < n; i += 32) __pipeline_memcpy_async(W.q + i + (size_t)c * ldq_s, gq + i + (size_t)c * n, sizeof(double));
         gcopy_async_wait();
@@ -1948,10 +1994,11 @@ hybrd_jac_kernel(SolverDev D, int cur, int per_group_doubles) {
         int *hi = (int *)W.scr;                            // [n + 1] last non-zero row per column (scr is free here)
         // Register-window accumulation of Q when the Jacobian at hand has the block-bidiagonal + border structure
         // (every sub-column fits the two-block window; fill-in stays inside it): decided per matrix, from its own zeros.
-        bool win = false;
+        // (the banded layout holds only for shapes whose every reflector fits the window, jac_band)
+        bool win = BAND;
         // (instantiated for the layout the 32 < P <= ~150 problems run with -- Q staged, R in global memory -- and the
         // block size of the benchmark model, 14; every other shape takes the barrier-per-reflector qform_g)
-        if ((G == 128) && STAGE_Q && !STAGE_R && D.N == 14 && n < G) {
+        if ((G == 128) && STAGE_Q && !STAGE_R && !BAND && D.N == 14 && n < G) {
             for (int k = tid; k < n; k += G) {
                 const double *ck = W.q + (size_t)k * W.ldq;
                 int last = 0;
@@ -1960,7 +2007,9 @@ hybrd_jac_kernel(SolverDev D, int cur, int per_group_doubles) {
             }
             win = window_ok<G>(n, D.N, hi, (int *)red);
         }
-        qrfac_g<G>(n, W.q, W.ldq, W.wa1, W.wa2, W.qtf, red, seq_warp<G>(D.sm_count), hi);
+        const DenseCols dense{W.q, W.ldq, n};
+        if constexpr (BAND) qrfac_g<G>(n, band, W.wa1, W.wa2, W.qtf, red, seq_warp<G>(D.sm_count), hi);
+        else qrfac_g<G>(n, dense, W.wa1, W.wa2, W.qtf, red, seq_warp<G>(D.sm_count), hi);
         SOCP_PHASE(32, 1);
         if (is[I_ITER] == 1) {
             for (int j = tid; j < n; j += G) {
@@ -1976,13 +2025,18 @@ hybrd_jac_kernel(SolverDev D, int cur, int per_group_doubles) {
             gsync<G>();
             if (tid == 0) { ds[D_XNORM] = xnorm; ds[D_DELTA] = delta; }
         }
-        pack_r_g<G>(n, W.q, W.ldq, W.wa1, W.r);
+        if constexpr (BAND) pack_r_g<G>(n, band, W.wa1, W.r);
+        else pack_r_g<G>(n, dense, W.wa1, W.r);
         SOCP_PHASE(32, 2);
         // register-window accumulation of Q when every reflector fits the two-block window (checked on this matrix):
         // no barrier, Q goes straight to global memory
         bool q_in_global = false;
-        if ((G == 128) && STAGE_Q && !STAGE_R && win) {
-            qform_p<G, 14>(n, W.q, W.ldq, hi, gq);
+        if constexpr (BAND) {
+            qform_p<G, 14>(n, band, hi, gq);
+            gsync<G>();
+            q_in_global = true;
+        } else if ((G == 128) && STAGE_Q && !STAGE_R && win) {
+            qform_p<G, 14>(n, dense, hi, gq);
             gsync<G>();
             q_in_global = true;
         } else qform_g<G>(n, W.q, W.ldq, W.wa1, seq_warp<G>(D.sm_count), hi);
@@ -2009,6 +2063,22 @@ hybrd_jac_kernel(SolverDev D, int cur, int per_group_doubles) {
         SOCP_PHASE(32, 6);
     }
     if (bulk && threadIdx.x == 0) bulk_wait_all();
+}
+
+template <int G, bool STAGE_R, bool STAGE_Q>
+__global__ void __launch_bounds__(128, 3)      // three CTAs per SM is what shared memory allows at P = 85: 168 registers
+hybrd_jac_kernel(SolverDev D, int cur, int per_group_doubles) {
+    jac_loop<G, STAGE_R, STAGE_Q, false>(D, cur, per_group_doubles);
+}
+
+// The Jacobian phase of the shapes with a structural band (SolverDev::band_doubles > 0, 32 < P <= 96, blocks of 14):
+// three warps, one thread per column, and the band instead of the dense matrix in shared memory (P = 85: 41 740 B instead
+// of 72 160 B per problem), so that five problems share an SM.  At five CTAs (15 warps, four on one SM sub-partition)
+// the register cap is 128: the kernel spills 96 bytes, of indices and pointers that stay fixed over a problem.
+// Four CTAs at 168 registers do not spill but were no faster than the dense kernel over a whole solve.
+__global__ void __launch_bounds__(96, 5)
+hybrd_jac_band_kernel(SolverDev D, int cur, int per_group_doubles) {
+    jac_loop<96, false, true, true>(D, cur, per_group_doubles);
 }
 
 // ---- small kernels -------------------------------------------------------------------------------
