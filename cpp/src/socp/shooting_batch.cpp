@@ -1,5 +1,5 @@
 // cpp/src/socp/shooting_batch.cpp -- see shooting_batch.hpp.  Host bookkeeping only; the numerical
-// work is socp_traj_batch / socp_solve_batch / socp_continuation_*_batch / socp_move_batch /
+// work is socp_init_shooting_batch / socp_solve_batch / socp_continuation_*_batch / socp_move_batch /
 // socp_solution_batch / socp_solution_trace_batch (include/socp_b200.h).
 #include <cstdlib>
 #include <cstring>
@@ -132,39 +132,26 @@ std::vector<real> shooting_batch::GetModelParameters(long k) const {
 void shooting_batch::InitShooting(std::vector<real> const& ti, std::vector<model::mstate> const& Xi,
                                   std::vector<real> const& tf, std::vector<model::mstate> const& Xf) {
 	const long B = data->B;
-	const int M = data->numMulti, n = data->dim, N = 2 * n, P = data->numParam, nodes = M + 1;
-	std::vector<real> X0((size_t)B * N), tnode(B), Xnode((size_t)B * N);
+	const int n = data->dim, N = 2 * n, P = data->numParam, np = data->np;
+	const size_t nodes = data->numMulti + 1;
+	std::vector<real> X0((size_t)B * N), XM((size_t)B * n), sw((size_t)B * 2);
+	// the switching times model::ComputeTraj integrates with (model.cpp:105-106)
+	const std::vector<real> & st = myModel.deviceSwitchingTimes;
+	const real sw0 = st.size() >= 2 ? st[0] : 0.0227, sw1 = st.size() >= 2 ? st[1] : 0.08;
 	for (long k = 0; k < B; k++) {
-		for (int i = 0; i <= M; i++) {
-			const real t = ti[k] + i * (tf[k] - ti[k]) / M;
-			data->time[k * nodes + i] = data->timed[k * nodes + i] = data->time_prec[k * nodes + i] = t;
-		}
-		for (int j = 0; j < N; j++) X0[k * N + j] = Xi[k][j];
-		for (int j = 0; j < n; j++) {
-			data->X[(k * nodes) * n + j] = Xi[k][j];
-			data->X[(k * nodes + M) * n + j] = Xf[k][j];
-		}
-		for (int j = 0; j < N; j++) data->param[k * P + j] = Xi[k][j];
+		std::copy(Xi[k].begin(), Xi[k].begin() + N, X0.begin() + k * N);
+		std::copy(Xf[k].begin(), Xf[k].begin() + n, XM.begin() + k * n);
+		sw[2 * k] = sw0; sw[2 * k + 1] = sw1;
 	}
-	for (int i = 1; i < M; i++) {				// interior nodes: the guess integrated from ti (shooting.cpp:218-222)
-		for (long k = 0; k < B; k++) tnode[k] = data->time[k * nodes + i];
-		data_struct *d = data;
-		const int np = data->np;
-		data->for_each_block([&, d, np, N](socp_ctx *ctx, long lo, long hi) {
-			if (socp_traj_batch(ctx, d->shape.model_id, d->shape.step_nbr, hi - lo, d->mparams.data() + lo * np, nullptr,
-			                    ti.data() + lo, tnode.data() + lo, X0.data() + lo * N, Xnode.data() + lo * N, SOCP_HOST) != SOCP_OK)
-				fail(ctx, "socp_traj_batch");
-		});
-		for (long k = 0; k < B; k++) {
-			for (int j = 0; j < N; j++) data->param[k * P + N * i + j] = Xnode[k * N + j];
-			for (int j = 0; j < n; j++) data->X[(k * nodes + i) * n + j] = Xnode[k * N + j];
-		}
-	}
-	for (long k = 0; k < B; k++) {
-		int q = N * M;
-		for (int j = 0; j <= M; j++)
-			if (data->shape.mode_t[j] == model::FREE) data->param[k * P + q++] = data->time[k * nodes + j];
-	}
+	data_struct *d = data;
+	data->for_each_block([&, d](socp_ctx *ctx, long lo, long hi) {
+		if (socp_init_shooting_batch(ctx, &d->shape, hi - lo, d->mparams.data() + lo * np, sw.data() + 2 * lo, ti.data() + lo,
+		                             X0.data() + lo * N, tf.data() + lo, XM.data() + lo * n, d->time.data() + lo * nodes,
+		                             d->X.data() + lo * nodes * n, d->param.data() + lo * P, SOCP_HOST) != SOCP_OK)
+			fail(ctx, "socp_init_shooting_batch");
+	});
+	data->timed = data->time;
+	data->time_prec = data->time;
 	data->Xd = data->X;
 	data->X_prec = data->X;
 }

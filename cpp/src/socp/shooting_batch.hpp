@@ -3,8 +3,8 @@
 // Same vocabulary and semantics as `shooting` (shooting.hpp), with a leading problem index:
 // Resize / SetMode / InitShooting / SetDesiredState / SolveOCP / GetParameters, Move / GetSolution to
 // sample the solutions and re-mesh them, and Trace.  One call of SolveOCP is one socp_solve_batch (or one batched
-// continuation) over all B problems; one Move, GetSolution or Trace is one socp_move_batch / socp_solution_batch /
-// socp_solution_trace_batch.
+// continuation) over all B problems; one InitShooting(ti, Xi, tf, Xf), Move, GetSolution or Trace is one
+// socp_init_shooting_batch / socp_move_batch / socp_solution_batch / socp_solution_trace_batch.
 #include <vector>
 
 #include "model.hpp"
@@ -38,7 +38,8 @@ public:
 	std::vector<real> GetModelParameters(long k) const;
 
 	/// shooting::InitShooting(ti, Xi, tf, Xf) for every problem: uniform time grid, interior nodes by
-	/// integrating the guess forward (one batched trajectory call per interior node)
+	/// integrating the guess forward with the model's integrator and switching times, as model::ComputeTraj does
+	/// (one socp_init_shooting_batch per device)
 	void InitShooting(std::vector<real> const& ti, std::vector<model::mstate> const& Xi,
 	                  std::vector<real> const& tf, std::vector<model::mstate> const& Xf);
 	/// shooting::InitShooting(vt, vX) for problem k

@@ -15,7 +15,7 @@
  * or SOCP_DEVICE (device pointers on the context's device; results are ordered on the context
  * stream: socp_sync() before reading them from another stream).  The batched solves and continuations
  * block the calling host thread intermittently: the round loop reads device-side work counters every
- * few rounds to know when the last problem has retired; the trajectory / residual / Jacobian / Move / GetSolution / Trace calls only enqueue.  There is no CPU fallback: without a CUDA device
+ * few rounds to know when the last problem has retired; the trajectory / residual / Jacobian / InitShooting / Move / GetSolution / Trace calls only enqueue.  There is no CPU fallback: without a CUDA device
  * socp_create fails.
  *
  * Data layouts (all double unless noted, row-major, one problem after another):
@@ -239,6 +239,18 @@ int socp_solution_batch(socp_ctx *ctx, const socp_shape *shape, long B, const do
  * observer.  B == 0: nothing is done. */
 int socp_solution_trace_batch(socp_ctx *ctx, const socp_shape *shape, long B, const double *mparams, const double *time,
                               const double *x, double *rows, int *nrows, int mem);
+
+/* The initial guess of B new problems: shooting::InitShooting(ti, Xi, tf, Xf) (shooting.cpp:202-245).  ti, tf [B],
+ * Xi [B][2dim], Xf [B][dim], sw: optional [B][2] goddard switching times, as in socp_traj_batch.  Outputs the problem
+ * inputs of socp_solve_batch: time [B][M+1] with time[b][i] = ti + i * (tf - ti) / M for every i (node M too, not
+ * tf), Xb [B][M+1][dim] (node 0 = Xi[:dim], node M = Xf, interior nodes the first dim values of their state) and
+ * x [B][P]: node 0 = Xi, interior node i = the integration of (ti, Xi) to time[b][i] with the shape's integrator,
+ * then the FREE node times in node order.  An interior node is bit for bit the socp_traj_batch (with SOCP_DOPRI5,
+ * socp_traj_adaptive_batch) of (ti, Xi, time[b][i], sw, step_nbr).  B == 0: nothing is done; M == 1: no
+ * integration. */
+int socp_init_shooting_batch(socp_ctx *ctx, const socp_shape *shape, long B, const double *mparams, const double *sw,
+                             const double *ti, const double *Xi, const double *tf, const double *Xf,
+                             double *time, double *Xb, double *x, int mem);
 
 /* FP64 FMA peak of the device measured with a register-resident DFMA chain (GFLOP/s). */
 int socp_measure_fp64_peak(socp_ctx *ctx, double *gflops, double *sm_clock_mhz);

@@ -1,5 +1,5 @@
 // socp_b200/csrc/move.cuh -- shooting::Move(tf), shooting::GetSolution and shooting::Trace for a batch of solved
-// problems.
+// problems, and shooting::InitShooting(ti, Xi, tf, Xf) for a batch of new ones.
 //
 // Restates shooting::Move(tf) (src/socp/shooting.cpp:383-437; cpp/src/socp/shooting.cpp:146-160) and
 // shooting::UpdateSolution (:1462-1508): the state of a solution at time t is the integration of the shooting
@@ -121,6 +121,78 @@ solution_trace_kernel(MoveShape sh, long B, int R, const double *__restrict__ mp
     double X[N];
     for (int i = 0; i < N; ++i) X[i] = xb[N * j + i];
     nrows[w] = trace_traj<MODEL>(c, X, t1, t2, sh.S, rows + w * R * W, W);
+}
+
+// shooting::InitShooting(ti, Xi, tf, Xf) (src/socp/shooting.cpp:202-245; cpp/src/socp/shooting.cpp:118-127): node i of
+// the uniform grid, with the reference's expression, so node M is this value and not tf.
+SOCP_DEV double init_node_time(double ti, double tf, int i, int M) { return ti + i * (tf - ti) / M; }
+
+// The time line and the copies of InitShooting: time[b] = the grid, node 0 = Xi[b] (x and Xb), Xb node M = Xf[b], and
+// the FREE node times after the node blocks of x[b], in node order.  One thread per output value: per problem, M + 1
+// times, N values of node 0, dim of node M, nfree times.  (One warp per problem, a lane per value, was measured slower:
+// 47 against 29 us for 10^5 Goddard problems on a B200 at its 1000 W power limit.)
+__global__ void __launch_bounds__(256)
+init_copies_kernel(MoveShape sh, long B, int n, const double *__restrict__ ti, const double *__restrict__ Xi,
+                   const double *__restrict__ tf, const double *__restrict__ Xf, double *__restrict__ time,
+                   double *__restrict__ Xb, double *__restrict__ x) {
+    const int N = 2 * n, nt = sh.M + 1, nfree = sh.P - N * sh.M;
+    const int per = nt + N + n + nfree;
+    for (long w = (long)blockIdx.x * blockDim.x + threadIdx.x; w < B * per; w += (long)gridDim.x * blockDim.x) {
+        const long b = w / per;
+        int r = (int)(w % per);
+        if (r < nt) {
+            time[b * nt + r] = init_node_time(ti[b], tf[b], r, sh.M);
+        } else if ((r -= nt) < N) {
+            const double v = Xi[b * N + r];
+            x[b * sh.P + r] = v;
+            if (r < n) Xb[b * nt * n + r] = v;
+        } else if ((r -= N) < n) {
+            Xb[(b * nt + sh.M) * n + r] = Xf[b * n + r];
+        } else {
+            r -= n;
+            int j = -1;                             // the node of the r-th FREE time
+            for (int k = 0; k <= r; ++k) do ++j; while (sh.mode_t[j] != SOCP_FREE);
+            x[b * sh.P + N * sh.M + r] = init_node_time(ti[b], tf[b], j, sh.M);
+        }
+    }
+}
+
+// Interior node i (1 <= i < M) of problem b: the integration of (ti[b], Xi[b]) to time[b][i], written to x[b][i] and its
+// first dim values to Xb[b][i]; time is init_copies_kernel's output.  compute_traj / compute_traj_adaptive with
+// traj_kernel's arguments, so a node is bit for bit the socp_traj_batch (socp_traj_adaptive_batch) of (ti, Xi, node time,
+// sw, S).  One work item per thread (group), node-major: blockIdx.y = i - 1, so the items of a warp share the interval
+// length (the adaptive step counts of a warp diverge less) and no thread divides its index by B.
+template <int MODEL, bool ADAPTIVE, int L = 1>
+__global__ void __launch_bounds__(SOCP_TRAJ_THREADS, Model<MODEL>::MINB)
+init_nodes_kernel(MoveShape sh, long B, const double *__restrict__ mparams, const double *__restrict__ sw,
+                  const double *__restrict__ ti, const double *__restrict__ Xi, const double *__restrict__ time,
+                  double *__restrict__ Xb, double *__restrict__ x, unsigned long long *counter) {
+    typedef Model<MODEL> M;
+    constexpr int N = M::N, n = M::DIM;
+    const int i = 1 + (int)blockIdx.y;
+    const int lane = (int)(threadIdx.x % L);
+    int steps = 0;
+    const long b = ((long)blockIdx.x * blockDim.x + threadIdx.x) / L;
+    if (b < B) {
+        typename M::Ctx c;
+        M::load(c, mparams + b * M::NP, sw ? sw + 2 * b : nullptr);
+        if (L > 1) Coop<MODEL>::set(c, lane);
+        double X[N];
+#pragma unroll
+        for (int k = 0; k < N; ++k) X[k] = Xi[b * N + k];
+        int st, rej = 0;
+        if (ADAPTIVE) st = compute_traj_adaptive<MODEL>(c, X, ti[b], time[b * (sh.M + 1) + i], sh.S, sh.ode_tol, rej);
+        else st = compute_traj<MODEL>(c, X, ti[b], time[b * (sh.M + 1) + i], sh.S);
+        if (lane == 0) {
+            double *xo = x + b * sh.P + (long)N * i, *Xo = Xb + (b * (sh.M + 1) + i) * n;
+#pragma unroll
+            for (int k = 0; k < N; ++k) xo[k] = X[k];
+#pragma unroll
+            for (int k = 0; k < n; ++k) Xo[k] = X[k];
+            steps += st;
+        }
+    }
+    count_steps(counter + (ADAPTIVE ? 3 : 0), steps);
 }
 
 }  // namespace socp

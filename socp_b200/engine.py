@@ -413,6 +413,35 @@ class Engine:
                                                       a.inp(x), a.out(rows), a.out(nrows, np.int32), mem))
         return rows, nrows
 
+    def init_shooting_batch(self, shape, mparams, ti, Xi, tf, Xf, sw=None):
+        """shooting::InitShooting(ti, Xi, tf, Xf) for B new problems of one shape (socp_init_shooting_batch): the
+        uniform time grid, node 0 = Xi, node M = Xf, every interior node integrated from (ti, Xi) with the shape's
+        integrator.  Xi is [B][2dim], Xf [B][dim], ti / tf [B], sw an optional [B][2] of goddard switching times.
+        Returns (time [B][M+1], Xb [B][M+1][dim], x [B][P]), the problem inputs of solve_batch.  Numpy arrays give numpy
+        results (scalar ti / tf and a 1-D mparams are broadcast); torch CUDA tensors give tensors on their device."""
+        M, dim, P = shape.num_multi, model_dim(shape.model_id), num_param(shape)
+        if P < 0:
+            raise ValueError("bad shape (model id / numMulti)")
+        mem = self._mem(Xi)
+        B = Xi.shape[0]
+        if mem == HOST:
+            Xi, Xf = np.asarray(Xi, dtype=np.float64), np.asarray(Xf, dtype=np.float64)
+            mparams = self._bcast_params(mparams, B, model_nparams(shape.model_id))
+            ti = np.broadcast_to(np.asarray(ti, dtype=np.float64), (B,))
+            tf = np.broadcast_to(np.asarray(tf, dtype=np.float64), (B,))
+            time, Xb, x = np.empty((B, M + 1)), np.empty((B, M + 1, dim)), np.empty((B, P))
+        else:
+            import torch
+            time = torch.empty((B, M + 1), dtype=torch.float64, device=Xi.device)
+            Xb = torch.empty((B, M + 1, dim), dtype=torch.float64, device=Xi.device)
+            x = torch.empty((B, P), dtype=torch.float64, device=Xi.device)
+        if tuple(Xi.shape) != (B, 2 * dim) or tuple(Xf.shape) != (B, dim):
+            raise ValueError("Xi must be [B][%d] and Xf [B][%d]" % (2 * dim, dim))
+        a = self._arg(mem)
+        self._check(self._L.socp_init_shooting_batch(self._h, ctypes.byref(shape), B, a.inp(mparams), a.inp(sw), a.inp(ti),
+                                                     a.inp(Xi), a.inp(tf), a.inp(Xf), a.out(time), a.out(Xb), a.out(x), mem))
+        return time, Xb, x
+
     # -- analytic-Jacobian path (modelOrder == 1; the double integrator, as in the reference) -----
     def traj_var_batch(self, model_id, mparams, t0, X0, tf, step_nbr=0):
         """model::ComputeTraj(isJac = 1) for B extended states [(2dim+1) 2dim] (host arrays)."""
